@@ -2,7 +2,7 @@
 """Benchmark of the per-timestep hot path: full-timestep Mcell-updates/s.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--scaling strong|weak]
-                    [--impl reference]
+                    [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the example loop body (reference ``examples/3d_examples/*``):
 ``dt = compute_stable_timestep()``, ``interactor()``, ``interactor.time_step(dt)``,
@@ -11,6 +11,11 @@ target (512^3 float32, flow_type "navier_stokes_with_forcing" with a virtual-bou
 forcing update + rotational-form update + diffusion + penalise + unbounded FFT Poisson + curl +
 immersed-boundary interpolation / spreading), strong-scaled over z-slabs for N > 1
 (BASELINE.json configs[4]).  One JSON line is printed by rank 0.
+
+The K timed steps always start from the synthetic initial condition, whatever number of warm-up steps
+it took to bring the clocks up, so that the same arguments compute the same steps.  ``--dump-outputs
+DIR`` (one process) writes what the last timed step handed its caller as ``DIR/<name>.npy``: see
+``dump_outputs``.
 """
 import argparse
 import json
@@ -342,9 +347,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-fused", action="store_true")
     ap.add_argument("--poisson-backend", type=str, default="auto")
+    ap.add_argument("--dump-outputs", type=str, default=None, metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (one process only)")
     ap.add_argument("--cpu-worker", type=str, default=None, help=argparse.SUPPRESS)
     ap.add_argument("--cpu-grid", type=str, default=None, help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path, not of --impl reference")
     if args.cpu_worker:
         cpu_oracle_worker(args.cpu_worker, tuple(int(v) for v in args.cpu_grid.split(",")), args.steps, args.warmup)
         return
@@ -367,6 +378,8 @@ def main():
     init_process_group_if_needed()
     world = dist.get_world_size() if dist.is_initialized() else 1
     rank = dist.get_rank() if dist.is_initialized() else 0
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs needs a single process (each rank only holds its own slab)")
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     torch.cuda.set_device(local_rank)
     device = torch.device("cuda", local_rank)
@@ -446,13 +459,19 @@ def main():
     for _ in range(int(extra.item())):
         one_step()
     n_warm += int(extra.item())
+    # back to the initial condition: how many warm-up steps ran depends on the speed of the build and
+    # of the GPU, what the timed steps compute must not
+    sim.vorticity_field[...] = host_w.to(device)
+    sim.compute_flow_velocity(free_stream_velocity=u_inf)
+    if interactor is not None:
+        interactor.global_lag_grid_position_mismatch_field = 0.0
     barrier()
     if sampler:
         sampler.mark()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record()
     for _ in range(args.steps):
-        one_step()
+        dt_last = one_step()
     ev1.record()
     barrier()
     ms_total = ev0.elapsed_time(ev1)
@@ -461,6 +480,8 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_step = t.item() / args.steps
     clocks = sampler.stop() if sampler else {}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, sim, interactor, dt_last)
 
     if os.environ.get("SB200_TRACE"):
         # developer aid: kernel-level timeline (CUPTI through torch.profiler) of three more steps, one
@@ -660,6 +681,47 @@ def main():
         torch.cuda.ipc_collect()
         dist.barrier()
         dist.destroy_process_group()
+
+
+DUMP_MAX_BYTES = 60 << 20  # with the .npy headers, under 64 MB in decimal units too
+DUMP_SEED = 0
+
+
+def dump_outputs(out_dir, sim, interactor, dt):
+    """What the last step handed its caller, as ``out_dir/<name>.npy`` (at most DUMP_MAX_BYTES in all):
+    ``dt`` (float64), the vorticity, velocity and stream-function fields as (3, n) arrays in the workload's
+    precision over the same n interior cells, and for workloads with a body the Lagrangian forcing and
+    position mismatch of every forcing point.  The cells are all interior cells when they fit, otherwise
+    a sample drawn with DUMP_SEED (sorted flat interior indices, z-major), so every run with the same
+    arguments writes the same cells."""
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"dt": np.array([float(dt)], dtype=np.float64)}
+    if interactor is not None:
+        out["lag_grid_forcing_field"] = np.array(interactor.global_lag_grid_forcing_field)
+        out["lag_grid_position_mismatch_field"] = np.array(interactor.global_lag_grid_position_mismatch_field)
+    fields = ("vorticity_field", "velocity_field", "stream_func_field")
+    gs = sim.ghost_size
+    padded = tuple(int(v) for v in sim.local_grid_size_with_ghost)
+    interior = tuple(v - 2 * gs for v in padded)
+    n_interior = int(np.prod(interior))
+    per_cell = len(fields) * 3 * np.dtype(sim.real_t).itemsize
+    n = (DUMP_MAX_BYTES - sum(a.nbytes for a in out.values())) // per_cell
+    if n >= n_interior:
+        cells = np.arange(n_interior)
+    else:
+        cells = np.unique(np.random.default_rng(DUMP_SEED).integers(0, n_interior, size=n))
+    zyx = np.unravel_index(cells, interior)
+    flat = np.ravel_multi_index(tuple(c + gs for c in zyx), padded)
+    import torch
+
+    index = torch.from_numpy(flat).to(sim.vorticity_field.tensor.device)
+    for name in fields:
+        t = getattr(sim, name).tensor
+        out[name] = t.reshape(t.shape[0], -1).index_select(1, index).cpu().numpy()
+    total = sum(a.nbytes for a in out.values())
+    assert total <= DUMP_MAX_BYTES and all(a.dtype in (np.float32, np.float64) for a in out.values()), total
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def count_launches(sim, interactor, u_inf, substeps=0):

@@ -6,6 +6,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
 
 
@@ -60,3 +62,44 @@ def test_importing_bench_leaves_stdout_alone(capfd):
     print("still here")
     out, _ = capfd.readouterr()
     assert "still here" in out
+
+
+def test_bench_rejects_bad_step_count_and_dump_of_reference_arm():
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True,
+                           timeout=120)
+        assert r.returncode == 2 and r.stdout == "", (extra, r.stderr[-2000:])
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("workload", ["vortex_ring_128_f32", "rod_fsi_128x64x64_f32"])
+def test_dumped_outputs_do_not_depend_on_the_warmup(workload, tmp_path):
+    """--dump-outputs: the timed steps start from the initial condition whatever the warm-up, so two runs
+    with different --warmup write the same outputs (up to the order of the spreading's float atomics)."""
+    import numpy as np
+    import torch
+
+    if not torch.cuda.is_available():
+        pytest.skip("needs a GPU")
+    dumps = []
+    for warmup in (1, 4):
+        out = tmp_path / f"warmup{warmup}"
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", workload, "--steps", "3",
+                            "--warmup", str(warmup), "--no-cpu-baseline", "--dump-outputs", str(out)],
+                           capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-3000:]
+        line = json.loads([ln for ln in r.stdout.splitlines() if ln.strip()][-1])
+        assert line["steps"] == 3 and line["config"]["workload"] == workload
+        dumps.append({p.name: np.load(p) for p in sorted(out.iterdir())})
+    names = {"dt.npy", "vorticity_field.npy", "velocity_field.npy", "stream_func_field.npy"}
+    if workload.startswith("rod"):
+        names |= {"lag_grid_forcing_field.npy", "lag_grid_position_mismatch_field.npy"}
+    assert set(dumps[0]) == names == set(dumps[1])
+    assert sum(os.path.getsize(tmp_path / "warmup1" / n) for n in names) <= 64_000_000
+    for name in names:
+        a, b = dumps[0][name], dumps[1][name]
+        assert a.dtype in (np.float32, np.float64) and a.shape == b.shape and np.isfinite(a).all(), name
+        assert np.abs(a - b).max() <= 1e-5 * np.abs(b).max(), name
+    # a grid that fits the budget is written whole; 128^3 is sampled
+    n_cells = dumps[0]["vorticity_field.npy"].shape[1]
+    assert n_cells == 128 * 64 * 64 if workload.startswith("rod") else 10 ** 6 < n_cells < 128 ** 3
