@@ -13,8 +13,6 @@
 // next plane's omega/u are prefetched into registers while the current one is processed.
 #include "sb200_common.h"
 
-#include <cstdlib>
-
 template <int TY, int TX, int NT>
 struct FusedTile {
   static constexpr int P2 = TX + 4, R2 = (TY + 4) * P2;  // tile + halo 2
@@ -421,6 +419,30 @@ __global__ void __launch_bounds__(32 * R)
     sb_vorticity_fused_v2_body<R, false>(g, out, w, u, p, d, zchunk, z_begin, z_end, smem);
 }
 
+// z chunks of the marching kernels: a block marches zchunk + 4 planes (4 to prime the rings), and the grid
+// of tiles x chunks runs in waves of `resident` blocks; pick the chunk count that minimises
+// waves x (zchunk + 4), with chunks of at least 8 planes.  (6 chunks at 260^3 were 918 blocks = 2.07 waves
+// of 444: a third wave for 30 blocks.)
+struct SbZChunks {
+  int chunks, zchunk;
+};
+static SbZChunks sb_z_chunks(long long tiles, int nzr, long long resident) {
+  SbZChunks r{1, nzr};
+  long long best = -1;
+  for (int c = 1; c <= nzr; ++c) {
+    const int zc = (nzr + c - 1) / c;
+    if (zc < 8 && c > 1) break;
+    const int cc = (nzr + zc - 1) / zc;  // chunks actually needed for this chunk length
+    const long long waves = (tiles * cc + resident - 1) / resident;
+    const long long cost = waves * (zc + 4);
+    if (best < 0 || cost < best) {
+      best = cost;
+      r = SbZChunks{cc, zc};
+    }
+  }
+  return r;
+}
+
 template <int R>
 static int launch_fused_v2(const SbGeom& g, void* out, const void* w, const void* u, double p, double d,
                            int z0, int z1, void* stream) {
@@ -442,26 +464,9 @@ static int launch_fused_v2(const SbGeom& g, void* out, const void* w, const void
     resident = cached;
   }
 #endif
-  const int nzr = z1 - z0;  // planes to produce
-  int chunks = 1, zchunk = nzr;
-  {
-    long long best = -1;
-    const long long tiles = (long long)gx * gy;
-    for (int c = 1; c <= nzr; ++c) {
-      const int zc = (nzr + c - 1) / c;
-      if (zc < 8 && c > 1) break;
-      const int cc = (nzr + zc - 1) / zc;
-      const long long waves = (tiles * cc + resident - 1) / resident;
-      const long long cost = waves * (zc + 4);
-      if (best < 0 || cost < best) {
-        best = cost;
-        chunks = cc;
-        zchunk = zc;
-      }
-    }
-  }
-  SB_LAUNCH_COOP((sb_vorticity_fused_v2_kernel<R>), dim3(gx, gy, (unsigned)chunks), dim3(FV::NT), smem, stream, g,
-                 (float*)out, (const float*)w, (const float*)u, (float)p, (float)d, zchunk, z0, z1);
+  const SbZChunks zc = sb_z_chunks((long long)gx * gy, z1 - z0, resident);
+  SB_LAUNCH_COOP((sb_vorticity_fused_v2_kernel<R>), dim3(gx, gy, (unsigned)zc.chunks), dim3(FV::NT), smem, stream, g,
+                 (float*)out, (const float*)w, (const float*)u, (float)p, (float)d, zc.zchunk, z0, z1);
   SB_CHECK_LAUNCH("vorticity_fused_v2");
   return 0;
 }
@@ -472,9 +477,6 @@ static int launch_fused(const SbGeom& g, void* out, const void* w, const void* u
   using FT = FusedTile<TY, TX, NT>;
   const size_t smem = sizeof(T) * FT::ELEMS;
   const unsigned gx = (g.mx + TX - 1) / TX, gy = (g.my + TY - 1) / TY;
-  // z chunks: a block marches zchunk + 4 planes (4 to prime the rings), and the grid runs in waves of
-  // `resident` blocks; pick the chunk count that minimises waves x (zchunk + 4).  (6 chunks at 260^3
-  // were 918 blocks = 2.07 waves of 444: a third wave for 30 blocks.)
   SB_KERNEL_ATTR_SMEM((sb_vorticity_fused_kernel<T, TY, TX, NT>), smem);
   long long resident = 148 * 3;
 #ifndef SB200_EMU
@@ -490,26 +492,9 @@ static int launch_fused(const SbGeom& g, void* out, const void* w, const void* u
     resident = cached;
   }
 #endif
-  const int nzr = z1 - z0;  // planes to produce
-  int chunks = 1, zchunk = nzr;
-  {
-    long long best = -1;
-    const long long tiles = (long long)gx * gy;
-    for (int c = 1; c <= nzr; ++c) {
-      const int zc = (nzr + c - 1) / c;
-      if (zc < 8 && c > 1) break;
-      const int cc = (nzr + zc - 1) / zc;  // chunks actually needed for this chunk length
-      const long long waves = (tiles * cc + resident - 1) / resident;
-      const long long cost = waves * (zc + 4);
-      if (best < 0 || cost < best) {
-        best = cost;
-        chunks = cc;
-        zchunk = zc;
-      }
-    }
-  }
-  SB_LAUNCH_COOP((sb_vorticity_fused_kernel<T, TY, TX, NT>), dim3(gx, gy, (unsigned)chunks), dim3(NT), smem,
-                 stream, g, (T*)out, (const T*)w, (const T*)u, (T)p, (T)d, zchunk, z0, z1);
+  const SbZChunks zc = sb_z_chunks((long long)gx * gy, z1 - z0, resident);
+  SB_LAUNCH_COOP((sb_vorticity_fused_kernel<T, TY, TX, NT>), dim3(gx, gy, (unsigned)zc.chunks), dim3(NT), smem,
+                 stream, g, (T*)out, (const T*)w, (const T*)u, (T)p, (T)d, zc.zchunk, z0, z1);
   SB_CHECK_LAUNCH("vorticity_fused");
   return 0;
 }
@@ -526,15 +511,9 @@ extern "C" int sb200_vorticity_rhs_fused_3d_range(const sb200_grid_t* gr, void* 
   SB_REQUIRE(z_begin >= 0 && z_end <= g.mz, "vorticity_rhs_fused_3d: bad plane range");
   if (z_end <= z_begin) return 0;
   if (gr->dtype == SB200_F32) {
-    // version 2 needs even row lengths (8-byte strips); SB200_FUSED_V2 = 0 / rows selects for measurements
-    static const int v2 = getenv("SB200_FUSED_V2") ? atoi(getenv("SB200_FUSED_V2")) : 24;
-    if (v2 > 0 && (g.mx & 1) == 0) {
-      if (v2 == 16)
-        return launch_fused_v2<16>(g, out, vorticity, velocity, curl_prefactor, nu_dt_by_dx2, z_begin, z_end, stream);
-      if (v2 == 20)
-        return launch_fused_v2<20>(g, out, vorticity, velocity, curl_prefactor, nu_dt_by_dx2, z_begin, z_end, stream);
+    // version 2 (24 rows per block) needs even row lengths (8-byte strips)
+    if ((g.mx & 1) == 0)
       return launch_fused_v2<24>(g, out, vorticity, velocity, curl_prefactor, nu_dt_by_dx2, z_begin, z_end, stream);
-    }
     // 16 x 32 tiles, 256 threads (version 1): measured best of 8x64, 12x32, 24x32, 16x48, 16x16 in round 1
     return launch_fused<float, 16, 32, 256>(g, out, vorticity, velocity, curl_prefactor, nu_dt_by_dx2, z_begin, z_end,
                                             stream);

@@ -34,11 +34,8 @@
 
 // A batch of lines.  Line (i, o1, o2) starts at element
 //     i + (o1 & (2^o1_shift - 1)) * s1 + (o1 >> o1_shift) * s1_hi + o2 * s2
-// and point k = t + p*Tn of it (p = 0..15) lives a further
-//     (p >> qs) * bstride + (t + (p & (2^qs - 1)) * Tn) * pt
-// elements on: with qs = 4 this is the plain "k * pt"; smaller qs splits the line into
-// 16 >> qs blocks of (2^qs * Tn) points that sit `bstride` apart (blocked layouts: TLB-friendly
-// z lines on one GPU, and the per-destination blocks of the slab transposes on several).
+// and point k of it lives a further k * pt elements on.  o1_shift / s1_hi split the o1 axis into
+// blocks (the per-source-rank blocks of the slab transposes); the default o1_shift = 30 is one block.
 // The grid is (ceil(inner / lines_per_block), n1, n2): no index division.
 struct SbLines {
   int inner, n1, n2;
@@ -46,8 +43,6 @@ struct SbLines {
   long long pt;
   int o1_shift = 30;
   long long s1_hi = 0;
-  int qs = 4;
-  long long bstride = 0;
   // grouped lines (tile-contiguous layout of the fused z pass): line i sits at (i & (2^gsh - 1)) inside
   // group i >> gsh, groups are s_grp elements apart.  gsh = 31: plain (line i at element i).
   int gsh = 31;
@@ -58,15 +53,6 @@ struct SbLines {
   SB_HD long long base(int i, int o1, int o2) const {
     return ((i + ((o1 >> 1) & rot)) & ((1u << gsh) - 1)) + (long long)(i >> gsh) * s_grp +
            (long long)(o1 & ((1 << o1_shift) - 1)) * s1 + (long long)(o1 >> o1_shift) * s1_hi + o2 * s2;
-  }
-  SB_HD long long point(int t, int p, int Tn) const {
-    return (long long)(p >> qs) * bstride + (long long)(t + (p & ((1 << qs) - 1)) * Tn) * pt;
-  }
-  // the same line seen by n / 32 threads of 32 points: point k = t + p Tn32 with Tn32 = Tn16 / 2, so
-  // a block of 2^qs sixteen-point slots holds 2^(qs+1) of these
-  SB_HD long long point32(int t, int p, int Tn) const {
-    const int q = qs + 1;
-    return (long long)(p >> q) * bstride + (long long)(t + (p & ((1 << q) - 1)) * Tn) * pt;
   }
 };
 
@@ -293,10 +279,9 @@ SB_D void sb_cp_async_wait_all() {
 }
 
 // specialised float kernels are held to <= 64 registers so that 1024 threads stay resident per SM.
-// BLOCKED = false: both line batches use the plain "k * pt" point addressing (qs == 4), so every
-// thread walks its 16 points with one running pointer (64-bit add per point, no multiplies).
-// VARIANT bit 0: blocked point addressing; bit 1: thread-order Green's table (gt.g2)
-template <typename T, int MODE, int LOG2N, int LINES, int VARIANT>
+// Every thread walks its 16 points with one running pointer (64-bit add per point, no multiplies).
+// G2: the fused pass scales by the thread-order Green's table (gt.g2) instead of the compressed one
+template <typename T, int MODE, int LOG2N, int LINES, bool G2>
 __global__ void __launch_bounds__(sb_lb_threads(LOG2N, LINES), MODE == 1 ? sb_lb_blocks_conv(LOG2N, LINES, sizeof(T)) : sb_lb_blocks(LOG2N, LINES, sizeof(T)))
     sb_fft_strided_kernel(SbFftPlan plan, int lb_shift_rt, const C2<T>* in, SbLines lin, C2<T>* out, SbLines lout,
                           const C2<T>* __restrict__ tw, SbGreensTable<T> gt) {
@@ -308,8 +293,6 @@ __global__ void __launch_bounds__(sb_lb_threads(LOG2N, LINES), MODE == 1 ? sb_lb
   const int l = threadIdx.x & ((1 << lb_shift) - 1), t = threadIdx.x >> lb_shift;
   // grid (kx group, o1, o2); the fused kernel with the thread-order table runs (o2, kx group, o1)
   // so that the components of one (kx, ky) tile are neighbours and share the table rows in L2
-  constexpr bool BLOCKED = (VARIANT & 1) != 0;
-  constexpr bool G2 = (VARIANT & 2) != 0;
   static_assert(!G2 || (MODE == 1 && LOG2N > 0 && sizeof(T) == 4), "thread-order table: fused float kernel");
   const int ib = G2 ? blockIdx.y : blockIdx.x;
   const int i = (ib << lb_shift) + l;
@@ -334,20 +317,15 @@ __global__ void __launch_bounds__(sb_lb_threads(LOG2N, LINES), MODE == 1 ? sb_lb
   C2<T> v[SB_FFT_R];
   {
     const C2<T>* gp = in + lin.base(ic, o1, o2);
-    if constexpr (BLOCKED) {
+    const long long sp = (long long)Tn * lin.pt;
+    gp += (long long)t * lin.pt;
 #pragma unroll
-      for (int p = 0; p < SB_FFT_R; ++p) v[p] = p < IN ? gp[lin.point(t, p, Tn)] : C2<T>{T(0), T(0)};
-    } else {
-      const long long sp = (long long)Tn * lin.pt;
-      gp += (long long)t * lin.pt;
-#pragma unroll
-      for (int p = 0; p < SB_FFT_R; ++p) {
-        if (p < IN) {
-          v[p] = *gp;
-          gp += sp;
-        } else {
-          v[p] = C2<T>{T(0), T(0)};
-        }
+    for (int p = 0; p < SB_FFT_R; ++p) {
+      if (p < IN) {
+        v[p] = *gp;
+        gp += sp;
+      } else {
+        v[p] = C2<T>{T(0), T(0)};
       }
     }
   }
@@ -394,94 +372,60 @@ __global__ void __launch_bounds__(sb_lb_threads(LOG2N, LINES), MODE == 1 ? sb_lb
   }
   if (valid) {
     C2<T>* gp = out + lout.base(i, o1, o2);
-    if constexpr (BLOCKED) {
+    const long long sp = (long long)Tn * lout.pt;
+    gp += (long long)t * lout.pt;
 #pragma unroll
-      for (int p = 0; p < OUT; ++p) gp[lout.point(t, p, Tn)] = v[p];
-    } else {
-      const long long sp = (long long)Tn * lout.pt;
-      gp += (long long)t * lout.pt;
-#pragma unroll
-      for (int p = 0; p < OUT; ++p) {
-        *gp = v[p];
-        gp += sp;
-      }
+    for (int p = 0; p < OUT; ++p) {
+      *gp = v[p];
+      gp += sp;
     }
   }
 }
 
 // ---------------------------------------------------------------- strided pass, 32 points per thread
 // Same passes (MODE 0 / 1 / 2) for n = 512 and 1024 with ONE shared-memory exchange per transform
-// (fft_device.h, sb_fft32_*): a line is n / 32 threads, a block 8 lines.  VARIANT as above
-// (bit 0 blocked point addressing, bit 1 thread-order Green's table with 32 factors per thread).
-constexpr int sb_p32_min_blocks(int mode, int log2n, int lines) {
+// (fft_device.h, sb_fft32_*): a line is n / 32 threads, a block 8 lines.  MODE 1 reads the compressed
+// Green's table: the 3D float z pass at these lengths is the fused z kernel below, so this one runs
+// the 2D y pass.
+constexpr int sb_p32_min_blocks(int log2n, int lines) {
   const int nt = lines * ((1 << log2n) / SB_FFT_P32);
-  if (mode == 2 && log2n == 9) return 768 / nt;  // the inverse-only pass fits 80 registers
-  return 512 / nt > 0 ? 512 / nt : 1;            // <= 128 registers per thread
+  return 512 / nt > 0 ? 512 / nt : 1;  // <= 128 registers per thread
 }
 
-template <typename T, int MODE, int LOG2N, int LINES, int VARIANT>
-__global__ void __launch_bounds__(LINES*((1 << LOG2N) / SB_FFT_P32), sb_p32_min_blocks(MODE, LOG2N, LINES))
+template <typename T, int MODE, int LOG2N, int LINES>
+__global__ void __launch_bounds__(LINES*((1 << LOG2N) / SB_FFT_P32), sb_p32_min_blocks(LOG2N, LINES))
     sb_fft_strided32_kernel(const C2<T>* in, SbLines lin, C2<T>* out, SbLines lout,
                             const C2<T>* __restrict__ tw, SbGreensTable<T> gt) {
   SB_DYN_SMEM(smem_raw);
   using FC = SbFft32C<LOG2N>;
-  constexpr int PT = SB_FFT_P32, Tn = FC::Tn, NT = LINES * Tn;
+  constexpr int PT = SB_FFT_P32, Tn = FC::Tn;
   constexpr int LINES_SHIFT = LINES == 16 ? 4 : LINES == 8 ? 3 : LINES == 4 ? 2 : LINES == 2 ? 1 : 0;
-  constexpr bool BLOCKED = (VARIANT & 1) != 0;
-  constexpr bool G2 = (VARIANT & 2) != 0;
-  static_assert(!G2 || (MODE == 1 && sizeof(T) == 4), "thread-order table: fused float kernel");
   constexpr int IN = (MODE == 0 || MODE == 1) ? PT / 2 : PT;
   constexpr int OUT = (MODE == 1 || MODE == 2) ? PT / 2 : PT;
   C2<T>* sm = reinterpret_cast<C2<T>*>(smem_raw);
   const int l = threadIdx.x & (LINES - 1), t = threadIdx.x >> LINES_SHIFT;
-  const int ib = G2 ? blockIdx.y : blockIdx.x;
-  const int i = (ib << LINES_SHIFT) + l;
-  const int o1 = G2 ? blockIdx.z : blockIdx.y, o2 = G2 ? blockIdx.x : blockIdx.z;
+  const int i = (blockIdx.x << LINES_SHIFT) + l;
+  const int o1 = blockIdx.y, o2 = blockIdx.z;
   const bool valid = i < lin.inner;
   const int ic = valid ? i : lin.inner - 1;
   C2<T>* sline = sm + l;
-  float4* gstage = nullptr;
-  if constexpr (G2) {
-    gstage = reinterpret_cast<float4*>(sm + LINES * FC::npad) + threadIdx.x;
-    const int g1 = o1 + gt.o1_off;
-    const int m1 = g1 <= (gt.n1_full >> 1) ? g1 : gt.n1_full - g1;
-    const float4* src = reinterpret_cast<const float4*>(gt.g2) +
-                        (((long long)m1 * gridDim.y + ib) * NT + threadIdx.x) * (PT / 4);
-#pragma unroll
-    for (int k = 0; k < PT / 4; ++k) sb_cp_async16(gstage + k * NT, src + k);
-  }
   C2<T> v[PT];
   {
     const C2<T>* gp = in + lin.base(ic, o1, o2);
-    if constexpr (BLOCKED) {
+    const long long sp = (long long)Tn * lin.pt;
+    gp += (long long)t * lin.pt;
 #pragma unroll
-      for (int p = 0; p < PT; ++p) v[p] = p < IN ? gp[lin.point32(t, p, Tn)] : C2<T>{T(0), T(0)};
-    } else {
-      const long long sp = (long long)Tn * lin.pt;
-      gp += (long long)t * lin.pt;
-#pragma unroll
-      for (int p = 0; p < PT; ++p) {
-        if (p < IN) {
-          v[p] = *gp;
-          gp += sp;
-        } else {
-          v[p] = C2<T>{T(0), T(0)};
-        }
+    for (int p = 0; p < PT; ++p) {
+      if (p < IN) {
+        v[p] = *gp;
+        gp += sp;
+      } else {
+        v[p] = C2<T>{T(0), T(0)};
       }
     }
   }
   if constexpr (MODE != 2) sb_fft32_forward_c<T, LOG2N, LINES, MODE == 1>(v, t, tw, sline);
-  if constexpr (G2) {
-    sb_cp_async_wait_all();
-#pragma unroll
-    for (int k = 0; k < PT / 4; ++k) {
-      const float4 gv = gstage[k * NT];
-      v[4 * k] = cscale(v[4 * k], gv.x);
-      v[4 * k + 1] = cscale(v[4 * k + 1], gv.y);
-      v[4 * k + 2] = cscale(v[4 * k + 2], gv.z);
-      v[4 * k + 3] = cscale(v[4 * k + 3], gv.w);
-    }
-  } else if constexpr (MODE == 1) {
+  if constexpr (MODE == 1) {
     const int g1 = o1 + gt.o1_off;
     const int m1 = g1 <= (gt.n1_full >> 1) ? g1 : gt.n1_full - g1;
     const int kxg = ic + gt.kx0 < gt.kx_last ? ic + gt.kx0 : gt.kx_last;
@@ -500,17 +444,12 @@ __global__ void __launch_bounds__(LINES*((1 << LOG2N) / SB_FFT_P32), sb_p32_min_
   if constexpr (MODE == 1 || MODE == 2) sb_fft32_inverse_c<T, LOG2N, LINES, false>(v, t, tw, sline);
   if (valid) {
     C2<T>* gp = out + lout.base(i, o1, o2);
-    if constexpr (BLOCKED) {
+    const long long sp = (long long)Tn * lout.pt;
+    gp += (long long)t * lout.pt;
 #pragma unroll
-      for (int p = 0; p < OUT; ++p) gp[lout.point32(t, p, Tn)] = v[p];
-    } else {
-      const long long sp = (long long)Tn * lout.pt;
-      gp += (long long)t * lout.pt;
-#pragma unroll
-      for (int p = 0; p < OUT; ++p) {
-        *gp = v[p];
-        gp += sp;
-      }
+    for (int p = 0; p < OUT; ++p) {
+      *gp = v[p];
+      gp += sp;
     }
   }
 }
@@ -541,19 +480,10 @@ SB_D void sb_bulk_load(void* smem_dst, const void* gsrc, unsigned bytes, unsigne
                "l"(gsrc), "r"(bytes), "r"(sb_smem_u32(bar))
                : "memory");
 }
-SB_D void sb_mbar_wait(unsigned long long* bar, unsigned parity) {
-  unsigned ok;
-  do {
-    asm volatile(
-        "{\n.reg .pred p;\nmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}"
-        : "=r"(ok)
-        : "r"(sb_smem_u32(bar)), "r"(parity)
-        : "memory");
-  } while (!ok);
-}
-// the same for a CONVERGED warp: the retry branch is taken on a warp vote, i.e. uniformly, so ptxas keeps
-// treating the warp as converged (a per-thread retry loop in front of a __syncwarp makes it emit the
-// out-of-line reconvergence path, with ~300 bytes of spills around it in the fused z kernel)
+// wait for phase `parity` of the barrier to complete, for a CONVERGED warp: the retry branch is taken on a
+// warp vote, i.e. uniformly, so ptxas keeps treating the warp as converged (a per-thread retry loop in front
+// of a __syncwarp makes it emit the out-of-line reconvergence path, with ~300 bytes of spills around it in
+// the fused z kernel)
 SB_D void sb_mbar_wait_warp(unsigned long long* bar, unsigned parity) {
   unsigned ok;
   do {
@@ -597,7 +527,6 @@ SB_D void sb_bulk_store(void* gdst, const void* smem_src, unsigned bytes) {
 }
 SB_D void sb_bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 SB_D void sb_bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-SB_D void sb_prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 #else
 // emulation: the barrier word is [completed phases : 32][bytes / 16 in flight : 16][arrival count : 8][pending : 8]
 SB_D void sb_mbar_init(unsigned long long* bar, unsigned count) {
@@ -627,81 +556,19 @@ SB_D void sb_bulk_load(void* smem_dst, const void* gsrc, unsigned bytes, unsigne
   sb_mbar_expect_if(true, bar, bytes);
   sb_bulk_copy_if(true, smem_dst, gsrc, bytes, bar);
 }
-SB_D void sb_mbar_wait(unsigned long long* bar, unsigned parity) {
+SB_D void sb_mbar_wait_warp(unsigned long long* bar, unsigned parity) {
   while (((__atomic_load_n(bar, __ATOMIC_SEQ_CST) >> 32) & 1u) == parity) std::this_thread::yield();
 }
-SB_D void sb_mbar_wait_warp(unsigned long long* bar, unsigned parity) { sb_mbar_wait(bar, parity); }
 SB_D void sb_fence_async_smem() { __atomic_thread_fence(__ATOMIC_SEQ_CST); }
 SB_D void sb_bulk_store(void* gdst, const void* smem_src, unsigned bytes) { memcpy(gdst, smem_src, bytes); }
 SB_D void sb_bulk_wait_read() {}
 SB_D void sb_bulk_wait_all() {}
-SB_D void sb_prefetch_l2(const void*) {}
 #endif
 
-constexpr int sb_zconv_blocks(int log2n) { return log2n >= 10 ? 2 : 4; }
-
-template <int LOG2N>
-__global__ void __launch_bounds__(8 * ((1 << LOG2N) / SB_FFT_P32), sb_zconv_blocks(LOG2N))
-    sb_fft_zconv32_kernel(C2<float>* B, int ntiles, int ncomp, int ng, int nky, const C2<float>* __restrict__ tw,
-                          const float* __restrict__ g2, int n1_full) {
-  using FC = SbFft32C<LOG2N>;
-  constexpr int PT = SB_FFT_P32, Tn = FC::Tn, LINES = 8, NT = LINES * Tn, NZ = FC::n / 2;
-  constexpr unsigned TILE = NZ * LINES;  // complex elements of a tile
-  SB_DYN_SMEM(smem_raw);
-  C2<float>* sm = reinterpret_cast<C2<float>*>(smem_raw);  // exchange buffer [npad][8]
-  C2<float>* sin = sm + LINES * FC::npad;                  // landing buffer of the tile [nz][8]
-  unsigned long long* bar = reinterpret_cast<unsigned long long*>(sin + TILE);
-  const int tid = threadIdx.x, l = tid & (LINES - 1), t = tid >> 3;
-  auto tile_offset = [&](int tile, int& kxg, int& ky) {
-    const int c = tile % ncomp, r = tile / ncomp;
-    kxg = r % ng;
-    ky = r / ng;
-    return (((long long)c * ng + kxg) * nky + ky) * (long long)TILE;
-  };
-  if (tid == 0) sb_mbar_init(bar, 1);
-  __syncthreads();
-  int tile = blockIdx.x, kxg = 0, ky = 0;
-  unsigned phase = 0;
-  if (tid == 0 && tile < ntiles) sb_bulk_load(sin, B + tile_offset(tile, kxg, ky), TILE * sizeof(C2<float>), bar);
-  __syncthreads();
-  for (; tile < ntiles; tile += gridDim.x) {
-    const long long off = tile_offset(tile, kxg, ky);
-    sb_mbar_wait(bar, phase);
-    phase ^= 1u;
-    C2<float> v[PT];
-#pragma unroll
-    for (int p = 0; p < PT; ++p)
-      v[p] = p < PT / 2 ? sin[(t + p * Tn) * LINES + l] : C2<float>{0.f, 0.f};
-    __syncthreads();  // the landing buffer has been consumed (and the previous tile's re-reads are done)
-    {
-      const int next = tile + gridDim.x;
-      int a, b;
-      if (tid == 0 && next < ntiles) sb_bulk_load(sin, B + tile_offset(next, a, b), TILE * sizeof(C2<float>), bar);
-    }
-    sb_fft32_forward_c<float, LOG2N, LINES, true>(v, t, tw, sm + l);
-    {
-      const int m1 = ky <= (n1_full >> 1) ? ky : n1_full - ky;
-      const float4* src = reinterpret_cast<const float4*>(g2) + (((long long)m1 * ng + kxg) * NT + tid) * (PT / 4);
-#pragma unroll
-      for (int k = 0; k < PT / 4; ++k) {
-        const float4 gv = src[k];
-        v[4 * k] = cscale(v[4 * k], gv.x);
-        v[4 * k + 1] = cscale(v[4 * k + 1], gv.y);
-        v[4 * k + 2] = cscale(v[4 * k + 2], gv.z);
-        v[4 * k + 3] = cscale(v[4 * k + 3], gv.w);
-      }
-    }
-    sb_fft32_inverse_c<float, LOG2N, LINES, false>(v, t, tw, sm + l);
-    C2<float>* out = B + off + (t * LINES + l);
-#pragma unroll
-    for (int p = 0; p < PT / 2; ++p) out[(long long)p * Tn * LINES] = v[p];
-  }
-}
-
 // ------------------------------------------------------ fused z pass, one line per warp
-// Same transform and tile layout as sb_fft_zconv32_kernel, organised so that no warp ever waits for
-// another one inside the transform (that kernel: 4 block barriers per tile, 2 resident blocks, FMA pipe
-// 56 % busy).  A line's n / 32 threads sit inside ONE warp (fft_device.h, sb_fft32w_forward), so:
+// A line's n / 32 threads sit inside ONE warp (fft_device.h, sb_fft32w_forward), so that no warp ever
+// waits for another one inside the transform: the kernel is bound by FP32 issue, and block barriers
+// between the exchange stages leave that pipe idle (DESIGN.md, "Fused z pass").  So:
 //   * the register-stage exchange is warp local (__syncwarp only);
 //   * a warp reads its line from the landed tile and writes the result back to the SAME slots: the tile
 //     buffer needs no block barrier either.  Reading column l of the [z][8] tile would be an 8- to 16-way
@@ -828,7 +695,8 @@ struct GreensExtractOp {
 };
 
 // compressed table g[mk][m1][kx] -> thread order g2[m1][ib][t][l][p]  (bin k = t + p Tn of the line
-// kx = ib LINES + l; mk = min(k, n - k)); kx beyond the pitch reads as zero
+// kx = ib LINES + l with 16 bins per thread, sb_fft_strided_kernel; mk = min(k, n - k)); kx beyond the
+// pitch reads as zero
 template <typename T>
 struct GreensThreadOrderOp {
   T* g2;
@@ -836,7 +704,6 @@ struct GreensThreadOrderOp {
   long long g_pt, g_s1;
   int n, Tn, lines, nib, pitch;
   int kx0, inner;  // first global kx of this rank's lines, number of lines
-  int pt;          // bins per thread (16 or 32)
   int warp_order = 0;  // 1: g5[m1][ib][l][n] (natural bin order per line, sb_fft_zconvw_kernel)
   SB_D void operator()(long long idx) const {
     int p, l, t;
@@ -851,8 +718,8 @@ struct GreensThreadOrderOp {
       g2[idx] = (i < inner && kx < pitch) ? g[mk * g_pt + m1 * g_s1 + kx] : T(0);
       return;
     } else {
-      p = (int)(idx % pt);
-      r = idx / pt;
+      p = (int)(idx % SB_FFT_R);
+      r = idx / SB_FFT_R;
       l = (int)(r % lines);
       r /= lines;
       t = (int)(r % Tn);
@@ -876,7 +743,6 @@ struct SbFftState {
   T* G2 = nullptr;     // thread-order copy of G for the specialised fused z kernel (float, 3D)
   long long P = 0;
   size_t bytes = 0;
-  int kb = 0;  // ky block size of the B layout (power of two, multiple of 2ny/16, divides 2ny)
   int kxl = 0; // x-slab decomposition: kx bins per rank (ceil((nx + 1) / nranks))
   // tile-contiguous layout of B + persistent bulk-copy z kernel (float, 3D, 2nz = 512 / 1024)
   bool zconv = false;
@@ -945,7 +811,7 @@ template <typename T, typename Rows, bool PRUNED>
 static int launch_x_r2c(const SbFftPlan& plan, int ny, int nz, int ncomp, const Rows& rows, C2<T>* out,
                         long long pitch, const C2<T>* tw, const C2<T>* wpost, void* stream,
                         const SbRowBlocks& rb = SbRowBlocks()) {
-  if (PRUNED) {  // compile-time specialised lengths, float and double
+  if constexpr (PRUNED) {  // compile-time specialised lengths, float and double
     switch (plan.log2n) {
       case 8: return launch_x_r2c_c<T, Rows, PRUNED, 8>(plan, ny, nz, ncomp, rows, out, pitch, tw, wpost, stream, rb);
       case 9: return launch_x_r2c_c<T, Rows, PRUNED, 9>(plan, ny, nz, ncomp, rows, out, pitch, tw, wpost, stream, rb);
@@ -985,13 +851,11 @@ static int launch_x_c2r(const SbFftPlan& plan, int ny, int nz, int ncomp, const 
   return launch_x_c2r_c<T, 0>(plan, ny, nz, ncomp, in, pitch, dst, tw, wpost, stream, rb);
 }
 
-// 32 points per thread (one exchange per transform) for n = 512 / 1024 in float; SB200_FFT_P32 is a
-// developer knob: bit m set = use it for MODE m (default below = what measured fastest on B200)
-static inline bool sb_use_p32(int mode, int log2n) {
-  // measured (profiles/r01_fft_tuning.md): n = 1024 all three passes, n = 512 the forward and the fused pass
-  static const int env = getenv("SB200_FFT_P32") ? atoi(getenv("SB200_FFT_P32")) : -1;
-  const int mask = env >= 0 ? env : (log2n == 10 ? 7 : 3);
-  return (log2n == 9 || log2n == 10) && mode >= 0 && mode <= 2 && ((mask >> mode) & 1);
+// 32 points per thread (one exchange per transform) for n = 512 / 1024 in float, in the passes where it
+// measured fastest on B200 (profiles/r01_fft_tuning.md): n = 1024 all three, n = 512 the forward and the
+// fused pass
+constexpr bool sb_use_p32(int mode, int log2n) {
+  return (log2n == 10 && mode <= 2) || (log2n == 9 && mode <= 1);
 }
 
 template <typename T, int MODE, int LOG2N>
@@ -999,32 +863,10 @@ static int launch_strided32(const C2<T>* in, const SbLines& lin, C2<T>* out, con
                             const C2<T>* tw, const SbGreensTable<T>& gt, void* stream) {
   constexpr int LINES = SB_P32_LINES(LOG2N), NT = LINES * ((1 << LOG2N) / SB_FFT_P32);
   const size_t smem = sizeof(C2<T>) * (size_t)LINES * SbFft32C<LOG2N>::npad;
-  const unsigned nib = (unsigned)((lin.inner + LINES - 1) / LINES);
-  const bool blocked = !(lin.qs == 4 && lout.qs == 4);
-#define SB_LAUNCH_STRIDED32(VARIANT, GRID, SMEM)                                                   \
-  do {                                                                                             \
-    SB_KERNEL_ATTR_SMEM((sb_fft_strided32_kernel<T, MODE, LOG2N, LINES, VARIANT>), SMEM);          \
-    SB_LAUNCH_COOP((sb_fft_strided32_kernel<T, MODE, LOG2N, LINES, VARIANT>), GRID, dim3(NT), SMEM, \
-                   stream, in, lin, out, lout, tw, gt);                                            \
-  } while (0)
-  if constexpr (MODE == 1) {
-    if (gt.g2) {
-      const size_t smem2 = smem + (size_t)NT * SB_FFT_P32 * sizeof(float);
-      const dim3 grid2((unsigned)lin.n2, nib, (unsigned)lin.n1);
-      if (blocked)
-        SB_LAUNCH_STRIDED32(3, grid2, smem2);
-      else
-        SB_LAUNCH_STRIDED32(2, grid2, smem2);
-      SB_CHECK_LAUNCH("fft_strided32");
-      return 0;
-    }
-  }
-  const dim3 grid(nib, (unsigned)lin.n1, (unsigned)lin.n2);
-  if (blocked)
-    SB_LAUNCH_STRIDED32(1, grid, smem);
-  else
-    SB_LAUNCH_STRIDED32(0, grid, smem);
-#undef SB_LAUNCH_STRIDED32
+  const dim3 grid((unsigned)((lin.inner + LINES - 1) / LINES), (unsigned)lin.n1, (unsigned)lin.n2);
+  SB_KERNEL_ATTR_SMEM((sb_fft_strided32_kernel<T, MODE, LOG2N, LINES>), smem);
+  SB_LAUNCH_COOP((sb_fft_strided32_kernel<T, MODE, LOG2N, LINES>), grid, dim3(NT), smem, stream, in, lin, out, lout,
+                 tw, gt);
   SB_CHECK_LAUNCH("fft_strided32");
   return 0;
 }
@@ -1033,53 +875,44 @@ template <typename T, int MODE, int LOG2N>
 static int launch_strided_c(const SbFftPlan& plan, const C2<T>* in, const SbLines& lin, C2<T>* out,
                             const SbLines& lout, const C2<T>* tw, const SbGreensTable<T>& gt, void* stream) {
   constexpr int LINES = LOG2N > 0 ? sb_strided_lines<T>(LOG2N, MODE) : 0;
-  if constexpr (sizeof(T) == 4 && (LOG2N == 9 || LOG2N == 10) && MODE <= 2) {
-    if (sb_use_p32(MODE, LOG2N)) return launch_strided32<T, MODE, LOG2N>(in, lin, out, lout, tw, gt, stream);
-  }
-  const int lb = LOG2N > 0 ? LINES : lines_per_block_for(plan.threads, sizeof(T), true);
-  const size_t smem = (size_t)lb * sb_fft_npad(plan.n) * sizeof(C2<T>);
-  int lb_shift = 0;
-  while ((1 << lb_shift) < lb) ++lb_shift;
-  const unsigned nib = (unsigned)((lin.inner + lb - 1) / lb);
-  const dim3 grid(nib, (unsigned)lin.n1, (unsigned)lin.n2);
-  const bool blocked = !(lin.qs == 4 && lout.qs == 4);
-#define SB_LAUNCH_STRIDED(VARIANT, GRID, SMEM)                                                             \
-  do {                                                                                                     \
-    SB_KERNEL_ATTR_SMEM((sb_fft_strided_kernel<T, MODE, LOG2N, LINES, VARIANT>), SMEM);                    \
-    SB_LAUNCH_COOP((sb_fft_strided_kernel<T, MODE, LOG2N, LINES, VARIANT>), GRID, dim3(lb * plan.threads), \
-                   SMEM, stream, plan, lb_shift, in, lin, out, lout, tw, gt);                              \
-  } while (0)
-  if constexpr (MODE == 1 && LOG2N > 0 && sizeof(T) == 4) {
-    if (gt.g2) {
-      // + 64 bytes per thread of staged Green's factors; grid (component, kx group, o1)
-      const size_t smem2 = smem + (size_t)lb * plan.threads * 64;
-      const dim3 grid2((unsigned)lin.n2, nib, (unsigned)lin.n1);
-      if (blocked)
-        SB_LAUNCH_STRIDED(3, grid2, smem2);
-      else
-        SB_LAUNCH_STRIDED(2, grid2, smem2);
-      SB_CHECK_LAUNCH("fft_strided");
-      return 0;
+  if constexpr (sizeof(T) == 4 && sb_use_p32(MODE, LOG2N)) {
+    return launch_strided32<T, MODE, LOG2N>(in, lin, out, lout, tw, gt, stream);
+  } else {
+    const int lb = LOG2N > 0 ? LINES : lines_per_block_for(plan.threads, sizeof(T), true);
+    const size_t smem = (size_t)lb * sb_fft_npad(plan.n) * sizeof(C2<T>);
+    int lb_shift = 0;
+    while ((1 << lb_shift) < lb) ++lb_shift;
+    const unsigned nib = (unsigned)((lin.inner + lb - 1) / lb);
+    if constexpr (MODE == 1 && LOG2N > 0 && sizeof(T) == 4) {
+      if (gt.g2) {
+        // + 64 bytes per thread of staged Green's factors; grid (component, kx group, o1)
+        const size_t smem2 = smem + (size_t)lb * plan.threads * 64;
+        const dim3 grid2((unsigned)lin.n2, nib, (unsigned)lin.n1);
+        SB_KERNEL_ATTR_SMEM((sb_fft_strided_kernel<T, MODE, LOG2N, LINES, true>), smem2);
+        SB_LAUNCH_COOP((sb_fft_strided_kernel<T, MODE, LOG2N, LINES, true>), grid2, dim3(lb * plan.threads), smem2,
+                       stream, plan, lb_shift, in, lin, out, lout, tw, gt);
+        SB_CHECK_LAUNCH("fft_strided");
+        return 0;
+      }
     }
+    const dim3 grid(nib, (unsigned)lin.n1, (unsigned)lin.n2);
+    SB_KERNEL_ATTR_SMEM((sb_fft_strided_kernel<T, MODE, LOG2N, LINES, false>), smem);
+    SB_LAUNCH_COOP((sb_fft_strided_kernel<T, MODE, LOG2N, LINES, false>), grid, dim3(lb * plan.threads), smem, stream,
+                   plan, lb_shift, in, lin, out, lout, tw, gt);
+    SB_CHECK_LAUNCH("fft_strided");
+    return 0;
   }
-  if (blocked)
-    SB_LAUNCH_STRIDED(1, grid, smem);
-  else
-    SB_LAUNCH_STRIDED(0, grid, smem);
-#undef SB_LAUNCH_STRIDED
-  SB_CHECK_LAUNCH("fft_strided");
-  return 0;
 }
 template <typename T, int MODE>
 static int launch_strided(const SbFftPlan& plan, const C2<T>* in, const SbLines& lin, C2<T>* out,
                           const SbLines& lout, const C2<T>* tw, const SbGreensTable<T>& gt, void* stream) {
-  if (MODE != 3) {  // compile-time specialised lengths (float: 256..2048, double: 256..1024)
+  if constexpr (MODE != 3) {  // compile-time specialised lengths (float: 256..2048, double: 256..1024)
     switch (plan.log2n) {
       case 8: return launch_strided_c<T, MODE, 8>(plan, in, lin, out, lout, tw, gt, stream);
       case 9: return launch_strided_c<T, MODE, 9>(plan, in, lin, out, lout, tw, gt, stream);
       case 10: return launch_strided_c<T, MODE, 10>(plan, in, lin, out, lout, tw, gt, stream);
       case 11:
-        if (sizeof(T) == 4) return launch_strided_c<T, MODE, 11>(plan, in, lin, out, lout, tw, gt, stream);
+        if constexpr (sizeof(T) == 4) return launch_strided_c<T, MODE, 11>(plan, in, lin, out, lout, tw, gt, stream);
         break;
       default: break;
     }
@@ -1088,38 +921,8 @@ static int launch_strided(const SbFftPlan& plan, const C2<T>* in, const SbLines&
 }
 
 template <int LOG2N>
-static int launch_zconv32(C2<float>* B, int ncomp, int ng, int nky, const C2<float>* tw, const float* g2,
-                          int n1_full, void* stream) {
-  using FC = SbFft32C<LOG2N>;
-  constexpr int NT = 8 * FC::Tn;
-  const size_t smem = sizeof(C2<float>) * (size_t)(8 * FC::npad + 8 * (FC::n / 2)) + 16;
-  SB_KERNEL_ATTR_SMEM((sb_fft_zconv32_kernel<LOG2N>), smem);
-  const long long ntiles = (long long)ncomp * ng * nky;
-  long long resident = 148LL * sb_zconv_blocks(LOG2N);
-#ifndef SB200_EMU
-  {
-    static long long cached = 0;
-    if (cached == 0) {
-      int dev = 0, sms = 0, per_sm = 0;
-      cudaGetDevice(&dev);
-      cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, sb_fft_zconv32_kernel<LOG2N>, NT, smem);
-      cached = (long long)sms * (per_sm > 0 ? per_sm : 1);
-    }
-    resident = cached;
-  }
-#else
-  resident = 3;  // a few persistent "blocks", several tiles each
-#endif
-  const unsigned grid = (unsigned)(ntiles < resident ? ntiles : resident);
-  SB_LAUNCH_COOP((sb_fft_zconv32_kernel<LOG2N>), dim3(grid), dim3(NT), smem, stream, B, (int)ntiles, ncomp, ng, nky,
-                 tw, g2, n1_full);
-  SB_CHECK_LAUNCH("fft_zconv32");
-  return 0;
-}
-template <int LOG2N>
 static int launch_zconvw(C2<float>* B, int ncomp, int ng, int nky, const C2<float>* tw, const float* g3,
-                         int n1_full, int* tile_counter, void* stream, int reserve_sms = 0) {
+                         int n1_full, int* tile_counter, void* stream) {
   using Z = SbZw<LOG2N>;
   SB_REQUIRE(tile_counter != nullptr, "fft_zconvw: no tile counter");
   sb_memset_async(tile_counter, 0, sizeof(int), stream);
@@ -1136,13 +939,9 @@ static int launch_zconvw(C2<float>* B, int ncomp, int ng, int nky, const C2<floa
       cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, sb_fft_zconvw_kernel<LOG2N>, Z::NT, Z::smem);
       if (per_sm < 1) per_sm = 1;
     }
-    // distributed solves overlap the peer-memory exchange of the neighbouring component with this kernel:
-    // a persistent grid that fills every SM would keep the push kernel out until it ends, so a few SMs
-    // stay free there
-    resident = (long long)(sms - (reserve_sms < sms ? reserve_sms : 0)) * per_sm;
+    resident = (long long)sms * per_sm;
   }
 #else
-  (void)reserve_sms;
   resident = 3;  // a few persistent "blocks", several tiles each
 #endif
   const unsigned grid = (unsigned)(ntiles < resident ? ntiles : resident);
@@ -1151,22 +950,13 @@ static int launch_zconvw(C2<float>* B, int ncomp, int ng, int nky, const C2<floa
   SB_CHECK_LAUNCH("fft_zconvw");
   return 0;
 }
-// fused z kernel on the tile-contiguous layout: 0 off, 1 block-synchronous (sb_fft_zconv32_kernel),
-// 2 one line per warp (sb_fft_zconvw_kernel, default); SB200_ZCONV is a developer knob
-static inline int sb_zconv_mode() {
-  static const int mode = getenv("SB200_ZCONV") ? atoi(getenv("SB200_ZCONV")) : 2;
-  return mode;
-}
+// fused z pass on the tile-contiguous layout (float, 2nz = 512 / 1024: SbFftState::zconv)
 template <typename T>
 static int launch_zconv(int log2n, C2<T>* B, int ncomp, int ng, int nky, const C2<T>* tw, const T* g2, int n1_full,
-                        int* tile_counter, void* stream, int reserve_sms = 0) {
+                        int* tile_counter, void* stream) {
   if constexpr (sizeof(T) == 4) {
-    if (sb_zconv_mode() == 2) {
-      if (log2n == 9) return launch_zconvw<9>((C2<float>*)B, ncomp, ng, nky, (const C2<float>*)tw, (const float*)g2, n1_full, tile_counter, stream, reserve_sms);
-      if (log2n == 10) return launch_zconvw<10>((C2<float>*)B, ncomp, ng, nky, (const C2<float>*)tw, (const float*)g2, n1_full, tile_counter, stream, reserve_sms);
-    }
-    if (log2n == 9) return launch_zconv32<9>((C2<float>*)B, ncomp, ng, nky, (const C2<float>*)tw, (const float*)g2, n1_full, stream);
-    if (log2n == 10) return launch_zconv32<10>((C2<float>*)B, ncomp, ng, nky, (const C2<float>*)tw, (const float*)g2, n1_full, stream);
+    if (log2n == 9) return launch_zconvw<9>(B, ncomp, ng, nky, tw, g2, n1_full, tile_counter, stream);
+    if (log2n == 10) return launch_zconvw<10>(B, ncomp, ng, nky, tw, g2, n1_full, tile_counter, stream);
   }
   sb_set_error("fft_zconv: unsupported transform length");
   return -1;
@@ -1183,11 +973,6 @@ static int fft_create_t(sb200_poisson* p, void* stream) {
   SB_REQUIRE(nx <= 4096 && ny <= 2048 && nz <= 2048, "fft backend: grid too large for one line per block");
   st->P = nx + 2;
   const long long P = st->P;
-  st->kb = 2 * ny;  // plain layout on one GPU (measured: blocking the ky axis does not pay here)
-  if (const char* env = getenv("SB200_FFT_KB")) {
-    const int v = atoi(env);
-    if (v >= st->py.threads && v <= 2 * ny && (v & (v - 1)) == 0) st->kb = v;
-  }
   st->twx = make_twiddles<T>(nx, nx, (double)nx, stream);
   st->wpost = make_twiddles<T>(nx, nx, 2.0 * nx, stream);
   st->twy = make_twiddles<T>(2 * ny, 2 * ny, 2.0 * ny, stream);
@@ -1207,8 +992,7 @@ static int fft_create_t(sb200_poisson* p, void* stream) {
   {
     const int inner = p->nranks > 1 ? st->kxl : nx + 1;
     st->ng = (inner + 7) / 8;
-    st->zconv = sb_zconv_mode() != 0 && sizeof(T) == 4 && p->dim == 3 && (st->pz.log2n == 9 || st->pz.log2n == 10) &&
-                sb_use_p32(1, st->pz.log2n);
+    st->zconv = sizeof(T) == 4 && p->dim == 3 && (st->pz.log2n == 9 || st->pz.log2n == 10);
   }
   if (st->zconv) SB_REQUIRE(SB_DEV_ALLOC(st->tile_counter, 64), "fft backend: cannot allocate the tile counter");
   const size_t b_bytes = p->dim != 3 ? 0
@@ -1251,20 +1035,20 @@ static int fft_create_t(sb200_poisson* p, void* stream) {
   const long long hz1 = p->dim == 3 ? nz + 1 : 1;
   e = sb_launch_flat(hz1 * (ny + 1) * P, GreensExtractOp<T>{st->G, full, P, n2y, (long long)ny + 1, (T)scale},
                      stream, "greens_extract");
-  if (!e && p->dim == 3 && sizeof(T) == 4 && st->pz.log2n >= 8 && st->pz.log2n <= 11) {
-    // thread-order copy for the specialised fused z kernel
-    const int pt = sb_use_p32(1, st->pz.log2n) ? SB_FFT_P32 : SB_FFT_R;
-    const int lines = pt == SB_FFT_P32 ? SB_P32_LINES(st->pz.log2n) : sb_strided_lines<T>(st->pz.log2n, 1);
-    const int Tn = 2 * nz / pt;
-    const int inner = p->nranks > 1 ? st->kxl : nx + 1, kx0 = p->nranks > 1 ? p->rank * st->kxl : 0;
-    const int nib = (inner + lines - 1) / lines;
-    const bool line_order = st->zconv && sb_zconv_mode() == 2;
-    const long long count = (long long)(ny + 1) * nib * Tn * lines * pt;  // (both orders: n floats per line)
-    SB_REQUIRE(SB_DEV_ALLOC(st->G2, sizeof(T) * count), "fft backend: cannot allocate the thread-order table");
-    st->bytes += sizeof(T) * count;
-    e = sb_launch_flat(count, GreensThreadOrderOp<T>{st->G2, st->G, (long long)(ny + 1) * P, P, 2 * nz, Tn, lines,
-                                                     nib, (int)P, kx0, inner, pt, line_order},
-                       stream, "greens_thread_order");
+  if constexpr (sizeof(T) == 4) {
+    if (!e && p->dim == 3 && st->pz.log2n >= 8 && st->pz.log2n <= 11) {
+      // reordered copy for the fused z pass: line order for the z kernel (zconv), thread order for the
+      // strided kernel (16 bins per thread)
+      const int lines = st->zconv ? SB_P32_LINES(st->pz.log2n) : sb_strided_lines<T>(st->pz.log2n, 1);
+      const int inner = p->nranks > 1 ? st->kxl : nx + 1, kx0 = p->nranks > 1 ? p->rank * st->kxl : 0;
+      const int nib = (inner + lines - 1) / lines;
+      const long long count = (long long)(ny + 1) * nib * lines * 2 * nz;  // (both orders: n floats per line)
+      SB_REQUIRE(SB_DEV_ALLOC(st->G2, sizeof(T) * count), "fft backend: cannot allocate the thread-order table");
+      st->bytes += sizeof(T) * count;
+      e = sb_launch_flat(count, GreensThreadOrderOp<T>{st->G2, st->G, (long long)(ny + 1) * P, P, 2 * nz,
+                                                       2 * nz / SB_FFT_R, lines, nib, (int)P, kx0, inner, st->zconv},
+                         stream, "greens_thread_order");
+    }
   }
   SB_STREAM_SYNC(stream);
   sb_poisson_free_greens_lines(lines_dev);
@@ -1295,7 +1079,7 @@ static int fft_solve_t(sb200_poisson* p, void* solution, const void* rhs, int nc
       SbLines lb{nx + 1, nz, ncomp, 8, (long long)st->ng * NKY * tile, tile};
       lb.gsh = 3;
       lb.s_grp = NKY * tile;
-      lb.rot = sb_zconv_mode() == 2 ? 7 : 0;
+      lb.rot = 7;
       if ((e = launch_strided<T, 0>(st->py, st->A, la, st->B, lb, st->twy, none, stream))) return e;
       st->mark(2, stream);
       if ((e = launch_zconv<T>(st->pz.log2n, st->B, ncomp, st->ng, (int)NKY, st->twz, st->G2, 2 * ny, st->tile_counter, stream))) return e;
@@ -1303,22 +1087,14 @@ static int fft_solve_t(sb200_poisson* p, void* solution, const void* rhs, int nc
       if ((e = launch_strided<T, 2>(st->py, st->B, lb, st->A, la, st->twy, none, stream))) return e;
       st->mark(4, stream);
     } else {
-    // y forward: A[c][z][y][kx] -> B[c][kyb][z][ky_in][kx]  (ky = kyb*KB + ky_in, see SbLines)
-      const int KB = st->kb, Tny = st->py.threads;
-      int kb_shift = 0, q_shift = 0;
-      while ((1 << kb_shift) < KB) ++kb_shift;
-      while ((Tny << q_shift) < KB) ++q_shift;
+      // y forward: A[c][z][y][kx] -> B[c][z][ky][kx]
       const long long cstride = 2LL * nz * ny * P;
       SbLines la{nx + 1, nz, ncomp, (long long)ny * P, (long long)nz * ny * P, P};
-      SbLines lb{nx + 1, nz, ncomp, (long long)KB * P, cstride, P};
-      lb.qs = q_shift;
-      lb.bstride = (long long)nz * KB * P;
+      SbLines lb{nx + 1, nz, ncomp, 2LL * ny * P, cstride, P};
       if ((e = launch_strided<T, 0>(st->py, st->A, la, st->B, lb, st->twy, none, stream))) return e;
       st->mark(2, stream);
-      // z: forward, x Ghat, inverse, in place on B; lines (kx, ky, c), points KB*P apart
-      SbLines lz{nx + 1, 2 * ny, ncomp, P, cstride, (long long)KB * P};
-      lz.o1_shift = kb_shift;
-      lz.s1_hi = (long long)nz * KB * P;
+      // z: forward, x Ghat, inverse, in place on B; lines (kx, ky, c), points 2ny*P apart
+      SbLines lz{nx + 1, 2 * ny, ncomp, P, cstride, 2LL * ny * P};
       SbGreensTable<T> gt{st->G, (long long)(ny + 1) * P, P, 2 * ny, 0};
       gt.g2 = st->G2;
       if ((e = launch_strided<T, 1>(st->pz, st->B, lz, st->B, lz, st->twz, gt, stream))) return e;
@@ -1466,10 +1242,10 @@ static int slab_spectral_t(sb200_poisson* p, void* recv, int ncomp, void* stream
     SbLines lb{sp.kxl, p->nz, ncomp, 8, (long long)st->ng * NKY * tile, tile};
     lb.gsh = 3;
     lb.s_grp = NKY * tile;
-    lb.rot = sb_zconv_mode() == 2 ? 7 : 0;
+    lb.rot = 7;
     if ((e = launch_strided<T, 0>(st->py, (const C2<T>*)recv, sp.lr, st->B, lb, st->twy, none, stream))) return e;
-    static const int reserve = getenv("SB200_ZCONV_RESERVE_SMS") ? atoi(getenv("SB200_ZCONV_RESERVE_SMS")) : 0;
-    if ((e = launch_zconv<T>(st->pz.log2n, st->B, ncomp, st->ng, (int)NKY, st->twz, st->G2, 2 * p->ny, st->tile_counter, stream, reserve)))
+    if ((e = launch_zconv<T>(st->pz.log2n, st->B, ncomp, st->ng, (int)NKY, st->twz, st->G2, 2 * p->ny, st->tile_counter,
+                             stream)))
       return e;
     return launch_strided<T, 2>(st->py, st->B, lb, (C2<T>*)recv, sp.lr, st->twy, none, stream);
   }

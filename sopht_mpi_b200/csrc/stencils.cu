@@ -4,7 +4,6 @@
 #include "sb200_common.h"
 
 #include <cstdarg>
-#include <cstdlib>
 
 static thread_local char g_err[512] = "";
 void sb_set_error(const char* fmt, ...) {
@@ -620,72 +619,17 @@ extern "C" int sb200_clear_physical_ring(const sb200_grid_t* gr, void* field, in
 // physical.  There every cell is either "deep" (written by each stage's interior call and outside
 // the zeroed ring) or in the ring, so the chain of FilterStageOp collapses to
 //     a = deep ? Fx(f) : 0,  b = deep ? Fy(a) : 0,  c = deep ? Fz(b) : 0,  f -= c
-// with F the 1D kernel 0.25 (-in(+1) - in(-1) + 2 in) (laplacian_filter_mpi_3d.py:62-99,267-319).  A block
-// stages an (8+2) x (8+2) x (32+2) tile (16+2 in double) of the field in shared memory and applies the three stages
-// there: 2 W per cell and component instead of 8 W + a copy.  OUT OF PLACE (a block reads a halo of
-// cells that belong to its neighbours): the simulator alternates between its two vorticity
-// allocations.  The last component also leaves the reference's buffer contents behind
-// (filter_flux_buffer = field_buffer = c).
-template <typename T>
-__global__ void __launch_bounds__(256)
-    sb_filter_o1_mult_kernel(SbGeom g, T* __restrict__ out, const T* __restrict__ field, int ncomp,
-                             T* __restrict__ flux, T* __restrict__ buf) {
-  constexpr int TX = sizeof(T) == 4 ? 32 : 16, TY = 8, TZ = 8;  // (static shared memory: <= 48 KB)
-  constexpr int FX = TX + 2, FY = TY + 2, FZ = TZ + 2;
-  __shared__ T sf[FZ * FY * FX];
-  __shared__ T sa[FZ * FY * TX];
-  __shared__ T sb[FZ * TY * TX];
-  const int x0 = blockIdx.x * TX, y0 = blockIdx.y * TY;
-  const int nzt = (g.mz + TZ - 1) / TZ;
-  const int c = blockIdx.z / nzt, z0 = (blockIdx.z - c * nzt) * TZ;
-  const T* f = field + (long long)c * g.vol;
-  T* o = out + (long long)c * g.vol;
-  const int tid = threadIdx.x;
-  for (int i = tid; i < FZ * FY * FX; i += 256) {
-    const int lx = i % FX, r = i / FX, ly = r % FY, lz = r / FY;
-    const int x = x0 + lx - 1, y = y0 + ly - 1, z = z0 + lz - 1;
-    const bool in = x >= 0 && x < g.mx && y >= 0 && y < g.my && z >= 0 && z < g.mz;
-    sf[i] = in ? f[g.idx(z, y, x)] : T(0);
-  }
-  __syncthreads();
-  for (int i = tid; i < FZ * FY * TX; i += 256) {
-    const int lx = i % TX, r = i / TX, ly = r % FY, lz = r / FY;
-    const int x = x0 + lx, y = y0 + ly - 1, z = z0 + lz - 1;
-    const bool in = x < g.mx && y >= 0 && y < g.my && z >= 0 && z < g.mz;
-    const T* q = sf + (lz * FY + ly) * FX + lx + 1;
-    sa[i] = (in && g.deep(z, y, x)) ? T(0.25) * (-q[1] - q[-1] + T(2) * q[0]) : T(0);
-  }
-  __syncthreads();
-  for (int i = tid; i < FZ * TY * TX; i += 256) {
-    const int lx = i % TX, r = i / TX, ly = r % TY, lz = r / TY;
-    const int x = x0 + lx, y = y0 + ly, z = z0 + lz - 1;
-    const bool in = x < g.mx && y < g.my && z >= 0 && z < g.mz;
-    const T* q = sa + (lz * FY + ly + 1) * TX + lx;
-    sb[i] = (in && g.deep(z, y, x)) ? T(0.25) * (-q[TX] - q[-TX] + T(2) * q[0]) : T(0);
-  }
-  __syncthreads();
-  const bool last = c == ncomp - 1;
-  for (int i = tid; i < TZ * TY * TX; i += 256) {
-    const int lx = i % TX, r = i / TX, ly = r % TY, lz = r / TY;
-    const int x = x0 + lx, y = y0 + ly, z = z0 + lz;
-    if (x >= g.mx || y >= g.my || z >= g.mz) continue;
-    const T* q = sb + ((lz + 1) * TY + ly) * TX + lx;
-    const T cz = g.deep(z, y, x) ? T(0.25) * (-q[TY * TX] - q[-TY * TX] + T(2) * q[0]) : T(0);
-    const long long gi = g.idx(z, y, x);
-    o[gi] = sf[((lz + 1) * FY + ly + 1) * FX + lx + 1] - cz;
-    if (last) {  // (the reference copies the flux into field_buffer after every stage)
-      flux[gi] = cz;
-      buf[gi] = cz;
-    }
-  }
-}
-// The same filter as a z MARCH (round 2): a block owns an 8 x 32 (y, x) tile and walks along z.  The x and y
-// stages are in-plane, so per plane it stages the tile + 1 halo cell (10 x 34) in shared memory, forms
-// a = Fx(f) on 10 x 32 and b = Fy(a) for the thread's own cell; the z stage only needs b at the SAME (y, x)
-// one plane up and down, which the thread carries in registers together with f of the previous plane.
-// Every plane is read once (+ the in-plane halo, served by L2) instead of the 1.66 x of the 8 x 8 x 32
-// brick, with no index arithmetic inside the march; the next plane is prefetched into registers.
-// Same expressions in the same order as sb_filter_o1_mult_kernel: bit-identical results.
+// with F the 1D kernel 0.25 (-in(+1) - in(-1) + 2 in) (laplacian_filter_mpi_3d.py:62-99,267-319): 2 W per
+// cell and component instead of 8 W + a copy.  OUT OF PLACE (a block reads a halo of cells that belong to
+// its neighbours): the simulator alternates between its two vorticity allocations.  The last component
+// also leaves the reference's buffer contents behind (filter_flux_buffer = field_buffer = c).
+// The filter is a z MARCH: a block owns an 8 x 32 (y, x) tile and walks along z.  The x and y stages are
+// in-plane, so per plane it stages the tile + 1 halo cell (10 x 34) in shared memory, forms a = Fx(f) on
+// 10 x 32 and b = Fy(a) for the thread's own cell; the z stage only needs b at the SAME (y, x) one plane up
+// and down, which the thread carries in registers together with f of the previous plane.  Every plane is
+// read once (+ the in-plane halo, served by L2), with no index arithmetic inside the march; the next plane
+// is prefetched into registers.  The expressions and their order are those of the stage chain, so the
+// results are bit-identical to it.
 template <typename T>
 __global__ void __launch_bounds__(256)
     sb_filter_o1_mult_march_kernel(SbGeom g, T* __restrict__ out, const T* __restrict__ field, int ncomp,
@@ -773,26 +717,17 @@ __global__ void __launch_bounds__(256)
 template <typename T>
 static int launch_filter_o1_mult(const SbGeom& g, void* out, const void* field, int ncomp, void* flux, void* buf,
                                  void* stream) {
-  static const bool march = !(getenv("SB200_FILTER_MARCH") && atoi(getenv("SB200_FILTER_MARCH")) == 0);
-  if (march) {
-    // z chunks: enough blocks for ~8 waves of the 148 x 8 resident blocks, at least 16 planes per chunk
-    const long long tiles = (long long)((g.mx + 31) / 32) * ((g.my + 7) / 8) * ncomp;
-    int nzc = (int)((148LL * 8 * 8 + tiles - 1) / tiles);
-    if (nzc < 1) nzc = 1;
-    int zchunk = (g.mz + nzc - 1) / nzc;
-    if (zchunk < 16) zchunk = g.mz < 16 ? g.mz : 16;
-    nzc = (g.mz + zchunk - 1) / zchunk;
-    const dim3 grid((unsigned)((g.mx + 31) / 32), (unsigned)((g.my + 7) / 8), (unsigned)(nzc * ncomp));
-    SB_LAUNCH_COOP(sb_filter_o1_mult_march_kernel<T>, grid, dim3(256), 0, stream, g, (T*)out, (const T*)field, ncomp,
-                   (T*)flux, (T*)buf, zchunk);
-    SB_CHECK_LAUNCH("filter_o1_mult_march");
-    return 0;
-  }
-  constexpr int TX = sizeof(T) == 4 ? 32 : 16;
-  const dim3 grid((unsigned)((g.mx + TX - 1) / TX), (unsigned)((g.my + 7) / 8), (unsigned)(((g.mz + 7) / 8) * ncomp));
-  SB_LAUNCH_COOP(sb_filter_o1_mult_kernel<T>, grid, dim3(256), 0, stream, g, (T*)out, (const T*)field, ncomp,
-                 (T*)flux, (T*)buf);
-  SB_CHECK_LAUNCH("filter_o1_mult");
+  // z chunks: enough blocks for ~8 waves of the 148 x 8 resident blocks, at least 16 planes per chunk
+  const long long tiles = (long long)((g.mx + 31) / 32) * ((g.my + 7) / 8) * ncomp;
+  int nzc = (int)((148LL * 8 * 8 + tiles - 1) / tiles);
+  if (nzc < 1) nzc = 1;
+  int zchunk = (g.mz + nzc - 1) / nzc;
+  if (zchunk < 16) zchunk = g.mz < 16 ? g.mz : 16;
+  nzc = (g.mz + zchunk - 1) / zchunk;
+  const dim3 grid((unsigned)((g.mx + 31) / 32), (unsigned)((g.my + 7) / 8), (unsigned)(nzc * ncomp));
+  SB_LAUNCH_COOP(sb_filter_o1_mult_march_kernel<T>, grid, dim3(256), 0, stream, g, (T*)out, (const T*)field, ncomp,
+                 (T*)flux, (T*)buf, zchunk);
+  SB_CHECK_LAUNCH("filter_o1_mult_march");
   return 0;
 }
 

@@ -407,13 +407,15 @@ def test_slab_decomposed_poisson_pipeline(real_t, n, nranks):
         assert np.all(out[r][:, 0] == 7.0) and np.all(out[r][:, :, :, -1] == 7.0)  # ghosts untouched
 
 
-@pytest.mark.parametrize("real_t", [np.float64, np.float32], ids=["f64", "f32"])
-def test_pruned_fft_poisson_pipeline_2d(real_t):
+# (256, 16): 2 ny = 512 runs the y pass through the 32-points-per-thread kernel (sb_fft_strided32_kernel)
+@pytest.mark.parametrize("real_t, n", [(np.float64, (16, 32)), (np.float32, (16, 32)), (np.float32, (256, 16))],
+                         ids=["f64", "f32", "f32-ny256"])
+def test_pruned_fft_poisson_pipeline_2d(real_t, n):
     from emu_util import emu
     from oracle.poisson import UnboundedPoissonSolverOracle2D
 
     lib = emu()
-    gs, n = 2, (16, 32)
+    gs = 2
     rng = np.random.default_rng(0)
     h = ctypes.c_void_p()
     _lib.check(lib, lib.sb200_poisson_create(ctypes.byref(h), 2, _lib.dtype_code(real_t), 1, n[0], n[1], gs,
