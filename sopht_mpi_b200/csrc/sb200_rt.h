@@ -64,16 +64,21 @@ extern thread_local dim3 t_blockDim, t_gridDim;
 extern thread_local BlockCtx* t_ctx;
 extern thread_local unsigned t_linear_tid;
 void launch(dim3 grid, dim3 block, size_t smem, bool coop, const std::function<void()>& body);
+// Records the address of a launched kernel in the runtime's launch log (sb200_emu_launched_kernels).
+// Taking the address also gives every instantiation a symbol of its own where g++ inlines the call.
+// Weak: a runtime that keeps no launch log still links, and then nothing is recorded.
+__attribute__((weak)) void note_launch(const void* kernel);
 }  // namespace sbemu
 #define threadIdx (sbemu::t_threadIdx)
 #define blockIdx (sbemu::t_blockIdx)
 #define blockDim (sbemu::t_blockDim)
 #define gridDim (sbemu::t_gridDim)
 #define SB_DYN_SMEM(name) unsigned char* name = sbemu::t_ctx->dyn_smem.data()
+#define SB_EMU_NOTE_LAUNCH(kernel) (sbemu::note_launch ? sbemu::note_launch((const void*)&kernel) : void())
 #define SB_LAUNCH(kernel, grid, block, smem, stream, ...) \
-  sbemu::launch((grid), (block), (smem), false, [&]() { kernel(__VA_ARGS__); })
+  (SB_EMU_NOTE_LAUNCH(kernel), sbemu::launch((grid), (block), (smem), false, [&]() { kernel(__VA_ARGS__); }))
 #define SB_LAUNCH_COOP(kernel, grid, block, smem, stream, ...) \
-  sbemu::launch((grid), (block), (smem), true, [&]() { kernel(__VA_ARGS__); })
+  (SB_EMU_NOTE_LAUNCH(kernel), sbemu::launch((grid), (block), (smem), true, [&]() { kernel(__VA_ARGS__); }))
 #define SB_KERNEL_ATTR_SMEM(kernel, bytes) (0)
 
 static inline void __syncthreads() { sbemu::t_ctx->block_bar->arrive_and_wait(); }
