@@ -733,17 +733,47 @@ struct GreensThreadOrderOp {
 };
 
 // --------------------------------------------------------------------- host state
+// The kx side of a handle: where the x passes put their output and which kx lines the y / z passes
+// transform.  A single-GPU solve is the one-rank case: all nz planes, rows of nx + 1 bins with pitch nx + 2.
+// A z-slab rank r of P runs the x passes on its nz / P planes and writes each row as P blocks of kxl bins,
+// one per destination rank; after the all-to-all it owns kx bins [r kxl, (r + 1) kxl) of ALL planes,
+// blocked by source rank: R[zb][c][zl][y][kx].
+struct SbKxSide {
+  int planes;       // planes of the x passes
+  int inner;        // kx lines of the y / z passes
+  long long pitch;  // row pitch of the x-pass output and of B[c][nz][2ny][pitch]
+  SbRowBlocks rb;   // blocks of the x-pass rows (contiguous on a single GPU)
+  SbLines lx;       // the x-pass output as lines (kx, z, c) along y
+  int kx0;          // global kx of line 0 (column of the Green's table)
+};
+static SbKxSide sb_kx_side(const sb200_poisson* p, int ncomp) {
+  const int nranks = p->nranks, nz = p->dim == 3 ? p->nz : 1, ny = p->ny;
+  SbKxSide k;
+  k.planes = nz / nranks;
+  k.inner = nranks > 1 ? sb_slab_kxl(p->nx, nranks) : p->nx + 1;
+  k.pitch = nranks > 1 ? k.inner : p->nx + 2;
+  k.kx0 = nranks > 1 ? p->rank * k.inner : 0;
+  const long long blk = (long long)ncomp * k.planes * ny * k.pitch;  // one destination / source block
+  k.lx = SbLines{k.inner, nz, ncomp, ny * k.pitch, k.planes * ny * k.pitch, k.pitch};
+  if (nranks > 1) {
+    k.rb = sb_row_blocks(k.inner, blk);
+    k.lx.o1_shift = 0;
+    while ((1 << k.lx.o1_shift) < k.planes) ++k.lx.o1_shift;
+    k.lx.s1_hi = blk;
+  }
+  return k;
+}
+
 template <typename T>
 struct SbFftState {
   SbFftPlan px, py, pz;
   C2<T>*twx = nullptr, *twy = nullptr, *twz = nullptr, *wpost = nullptr;
-  C2<T>* A = nullptr;  // [ncomp][nz][ny][P]
-  C2<T>* B = nullptr;  // [ncomp][nz][2ny][P]
+  C2<T>* A = nullptr;  // [ncomp][nz][ny][P]  (single GPU)
+  C2<T>* B = nullptr;  // [ncomp][nz][2ny][pitch]  (SbKxSide)
   T* G = nullptr;      // [nz+1][ny+1][P]  (2D: [ny+1][P])
   T* G2 = nullptr;     // thread-order copy of G for the specialised fused z kernel (float, 3D)
   long long P = 0;
   size_t bytes = 0;
-  int kxl = 0; // x-slab decomposition: kx bins per rank (ceil((nx + 1) / nranks))
   // tile-contiguous layout of B + persistent bulk-copy z kernel (float, 3D, 2nz = 512 / 1024)
   bool zconv = false;
   int ng = 0;  // kx groups of 8 lines
@@ -984,21 +1014,14 @@ static int fft_create_t(sb200_poisson* p, void* stream) {
                "fft backend: slab decomposition needs 2, 4 or 8 ranks");
     SB_REQUIRE(nz % p->nranks == 0 && nz / p->nranks >= 2 * p->gs, "fft backend: nz must split into slabs");
   }
-  // distributed: the x-pass output goes straight into the caller's exchange buffer (blocked by
-  // destination rank); after the transpose this rank owns kxl kx bins of ALL planes and runs the
-  // y and z passes on B[c][nz][2ny][kxl]
-  st->kxl = p->nranks > 1 ? sb_slab_kxl(nx, p->nranks) : 0;
+  const SbKxSide kx = sb_kx_side(p, 3);
   const size_t a_bytes = p->nranks == 1 ? sizeof(C2<T>) * 3 * (size_t)(p->dim == 3 ? nz : 1) * ny * P : 0;
-  {
-    const int inner = p->nranks > 1 ? st->kxl : nx + 1;
-    st->ng = (inner + 7) / 8;
-    st->zconv = sizeof(T) == 4 && p->dim == 3 && (st->pz.log2n == 9 || st->pz.log2n == 10);
-  }
+  st->ng = (kx.inner + 7) / 8;
+  st->zconv = sizeof(T) == 4 && p->dim == 3 && (st->pz.log2n == 9 || st->pz.log2n == 10);
   if (st->zconv) SB_REQUIRE(SB_DEV_ALLOC(st->tile_counter, 64), "fft backend: cannot allocate the tile counter");
+  // B: tile-contiguous (zconv) or [c][nz][2ny][pitch]
   const size_t b_bytes = p->dim != 3 ? 0
-                         : st->zconv ? sizeof(C2<T>) * 3 * (size_t)nz * 2 * ny * 8 * st->ng
-                         : p->nranks == 1 ? sizeof(C2<T>) * 3 * (size_t)nz * 2 * ny * P
-                                          : sizeof(C2<T>) * 3 * (size_t)nz * 2 * ny * st->kxl;
+                         : sizeof(C2<T>) * 3 * (size_t)nz * 2 * ny * (st->zconv ? 8LL * st->ng : kx.pitch);
   const size_t g_bytes = sizeof(T) * (p->dim == 3 ? (nz + 1) : 1) * (ny + 1) * P;
   if (a_bytes) SB_REQUIRE(SB_DEV_ALLOC(st->A, a_bytes), "fft backend: cannot allocate x-pass buffer");
   if (b_bytes) SB_REQUIRE(SB_DEV_ALLOC(st->B, b_bytes), "fft backend: cannot allocate y-pass buffer");
@@ -1040,13 +1063,13 @@ static int fft_create_t(sb200_poisson* p, void* stream) {
       // reordered copy for the fused z pass: line order for the z kernel (zconv), thread order for the
       // strided kernel (16 bins per thread)
       const int lines = st->zconv ? SB_P32_LINES(st->pz.log2n) : sb_strided_lines<T>(st->pz.log2n, 1);
-      const int inner = p->nranks > 1 ? st->kxl : nx + 1, kx0 = p->nranks > 1 ? p->rank * st->kxl : 0;
-      const int nib = (inner + lines - 1) / lines;
+      const int nib = (kx.inner + lines - 1) / lines;
       const long long count = (long long)(ny + 1) * nib * lines * 2 * nz;  // (both orders: n floats per line)
       SB_REQUIRE(SB_DEV_ALLOC(st->G2, sizeof(T) * count), "fft backend: cannot allocate the thread-order table");
       st->bytes += sizeof(T) * count;
       e = sb_launch_flat(count, GreensThreadOrderOp<T>{st->G2, st->G, (long long)(ny + 1) * P, P, 2 * nz,
-                                                       2 * nz / SB_FFT_R, lines, nib, (int)P, kx0, inner, st->zconv},
+                                                       2 * nz / SB_FFT_R, lines, nib, (int)P, kx.kx0, kx.inner,
+                                                       st->zconv},
                          stream, "greens_thread_order");
     }
   }
@@ -1056,65 +1079,83 @@ static int fft_create_t(sb200_poisson* p, void* stream) {
   return e;
 }
 
+// ------------------------------------------ the three stages of a solve, single GPU and z-slab alike
+// X is the x-pass output: the buffer A of a single-GPU solve, the caller's exchange buffers of a z-slab
+// rank (SbKxSide).  Profiling marks 2 and 3 sit inside the spectral stage (they only record on a
+// single-rank handle).
+template <typename T>
+static FieldRows<T> sb_field_rows(const sb200_poisson* p, const SbKxSide& kx, const void* f) {
+  const long long my = p->ny + 2 * p->gs, mx = p->nx + 2 * p->gs;
+  const long long vol = (p->dim == 3 ? kx.planes + 2LL * p->gs : 1) * my * mx;
+  return FieldRows<T>{(T*)f, p->ny, p->gs, p->dim, my, mx, vol};
+}
+template <typename T>
+static int fft_x_forward_t(sb200_poisson* p, const void* rhs, int ncomp, C2<T>* X, void* stream) {
+  auto* st = (SbFftState<T>*)p->backend_state;
+  const SbKxSide kx = sb_kx_side(p, ncomp);
+  return launch_x_r2c<T, FieldRows<T>, true>(st->px, p->ny, kx.planes, ncomp, sb_field_rows<T>(p, kx, rhs), X,
+                                             kx.pitch, st->twx, st->wpost, stream, kx.rb);
+}
+template <typename T>
+static int fft_spectral_t(sb200_poisson* p, C2<T>* X, int ncomp, void* stream) {
+  auto* st = (SbFftState<T>*)p->backend_state;
+  const SbKxSide kx = sb_kx_side(p, ncomp);
+  const int nz = p->nz, ny = p->ny;
+  const long long P = st->P, pitch = kx.pitch;
+  SbGreensTable<T> none{nullptr, 0, 0};
+  SbGreensTable<T> gt{st->G, (p->dim == 3 ? ny + 1LL : 1LL) * P, P, 2 * ny, 0};
+  gt.g2 = st->G2;
+  gt.kx0 = kx.kx0;
+  gt.kx_last = (int)P - 1;
+  int e;
+  if (p->dim == 2) {  // fused forward / x Ghat / inverse along y, in place on X
+    st->mark(2, stream);
+    if ((e = launch_strided<T, 1>(st->py, X, kx.lx, X, kx.lx, st->twy, gt, stream))) return e;
+    st->mark(3, stream);
+    return 0;
+  }
+  // y forward X -> B, z pass in place on B, y inverse B -> X.  B is either tile-contiguous for the
+  // persistent z kernel, Bt[c][kx group][ky][z][8] addressed through grouped lines, or B[c][z][ky][pitch]
+  const long long nky = 2LL * ny, tile = (long long)nz * 8;
+  SbLines lb{kx.inner, nz, ncomp, nky * pitch, nz * nky * pitch, pitch};
+  if (st->zconv) {
+    lb = SbLines{kx.inner, nz, ncomp, 8, st->ng * nky * tile, tile};
+    lb.gsh = 3;
+    lb.s_grp = nky * tile;
+    lb.rot = 7;
+  }
+  if ((e = launch_strided<T, 0>(st->py, X, kx.lx, st->B, lb, st->twy, none, stream))) return e;
+  st->mark(2, stream);
+  if (st->zconv) {
+    e = launch_zconv<T>(st->pz.log2n, st->B, ncomp, st->ng, (int)nky, st->twz, st->G2, 2 * ny, st->tile_counter,
+                        stream);
+  } else {  // lines (kx, ky, c), points along z
+    SbLines lz{kx.inner, 2 * ny, ncomp, pitch, nz * nky * pitch, nky * pitch};
+    e = launch_strided<T, 1>(st->pz, st->B, lz, st->B, lz, st->twz, gt, stream);
+  }
+  if (e) return e;
+  st->mark(3, stream);
+  return launch_strided<T, 2>(st->py, st->B, lb, X, kx.lx, st->twy, none, stream);
+}
+template <typename T>
+static int fft_x_backward_t(sb200_poisson* p, void* solution, int ncomp, const C2<T>* X, void* stream) {
+  auto* st = (SbFftState<T>*)p->backend_state;
+  const SbKxSide kx = sb_kx_side(p, ncomp);
+  return launch_x_c2r<T>(st->px, p->ny, kx.planes, ncomp, X, kx.pitch, sb_field_rows<T>(p, kx, solution), st->twx,
+                         st->wpost, stream, kx.rb);
+}
+
 template <typename T>
 static int fft_solve_t(sb200_poisson* p, void* solution, const void* rhs, int ncomp, void* stream) {
   auto* st = (SbFftState<T>*)p->backend_state;
   SB_REQUIRE(ncomp >= 1 && ncomp <= 3, "poisson_solve: ncomp must be 1..3");
-  const int nz = p->dim == 3 ? p->nz : 1, ny = p->ny, nx = p->nx, gs = p->gs;
-  const long long P = st->P;
-  const long long my = ny + 2 * gs, mx = nx + 2 * gs;
-  const long long vol = (p->dim == 3 ? nz + 2LL * gs : 1) * my * mx;
   int e;
-  FieldRows<T> src{(T*)rhs, ny, gs, p->dim, my, mx, vol};
   st->mark(0, stream);
-  if ((e = launch_x_r2c<T, FieldRows<T>, true>(st->px, ny, nz, ncomp, src, st->A, P, st->twx, st->wpost, stream)))
-    return e;
+  if ((e = fft_x_forward_t<T>(p, rhs, ncomp, st->A, stream))) return e;
   st->mark(1, stream);
-  SbGreensTable<T> none{nullptr, 0, 0};
-  if (p->dim == 3) {
-    if (st->zconv) {
-      // tile-contiguous B: Bt[c][kx group][ky][z][8]; y passes address it through grouped lines
-      const long long NZ = nz, NKY = 2LL * ny, tile = NZ * 8;
-      SbLines la{nx + 1, nz, ncomp, (long long)ny * P, (long long)nz * ny * P, P};
-      SbLines lb{nx + 1, nz, ncomp, 8, (long long)st->ng * NKY * tile, tile};
-      lb.gsh = 3;
-      lb.s_grp = NKY * tile;
-      lb.rot = 7;
-      if ((e = launch_strided<T, 0>(st->py, st->A, la, st->B, lb, st->twy, none, stream))) return e;
-      st->mark(2, stream);
-      if ((e = launch_zconv<T>(st->pz.log2n, st->B, ncomp, st->ng, (int)NKY, st->twz, st->G2, 2 * ny, st->tile_counter, stream))) return e;
-      st->mark(3, stream);
-      if ((e = launch_strided<T, 2>(st->py, st->B, lb, st->A, la, st->twy, none, stream))) return e;
-      st->mark(4, stream);
-    } else {
-      // y forward: A[c][z][y][kx] -> B[c][z][ky][kx]
-      const long long cstride = 2LL * nz * ny * P;
-      SbLines la{nx + 1, nz, ncomp, (long long)ny * P, (long long)nz * ny * P, P};
-      SbLines lb{nx + 1, nz, ncomp, 2LL * ny * P, cstride, P};
-      if ((e = launch_strided<T, 0>(st->py, st->A, la, st->B, lb, st->twy, none, stream))) return e;
-      st->mark(2, stream);
-      // z: forward, x Ghat, inverse, in place on B; lines (kx, ky, c), points 2ny*P apart
-      SbLines lz{nx + 1, 2 * ny, ncomp, P, cstride, 2LL * ny * P};
-      SbGreensTable<T> gt{st->G, (long long)(ny + 1) * P, P, 2 * ny, 0};
-      gt.g2 = st->G2;
-      if ((e = launch_strided<T, 1>(st->pz, st->B, lz, st->B, lz, st->twz, gt, stream))) return e;
-      st->mark(3, stream);
-      // y inverse: B -> A
-      if ((e = launch_strided<T, 2>(st->py, st->B, lb, st->A, la, st->twy, none, stream))) return e;
-      st->mark(4, stream);
-    }
-  } else {
-    st->mark(2, stream);
-    // 2D: fused forward / multiply / inverse along y, in place on A; lines (kx, -, c)
-    SbLines ly{nx + 1, 1, ncomp, 0, (long long)ny * P, P};
-    SbGreensTable<T> gt{st->G, P, 0, 1, 0};
-    if ((e = launch_strided<T, 1>(st->py, st->A, ly, st->A, ly, st->twy, gt, stream))) return e;
-    st->mark(3, stream);
-    st->mark(4, stream);
-  }
-  FieldRows<T> dst{(T*)solution, ny, gs, p->dim, my, mx, vol};
-  e = launch_x_c2r<T>(st->px, ny, nz, ncomp, (const C2<T>*)st->A, P, dst, (const C2<T>*)st->twx,
-                      (const C2<T>*)st->wpost, stream);
+  if ((e = fft_spectral_t<T>(p, st->A, ncomp, stream))) return e;
+  st->mark(4, stream);
+  e = fft_x_backward_t<T>(p, solution, ncomp, st->A, stream);
   st->mark(5, stream);
   st->have_times = st->profile && e == 0;
   return e;
@@ -1191,83 +1232,9 @@ int sb_poisson_fft_create(sb200_poisson* p, void* stream) {
 //   spectral: y forward R -> B[c][z][ky][kx_in], fused z pass in place on B (Green's table columns
 //             kx0 + kx_in), y inverse B -> R (same blocked-by-z layout)
 //   all-to-all back, backward: x c2r of the local planes from S.
+// The three stages are the ones of the single-GPU solve (fft_solve_t) on the caller's buffers.
 // Bins beyond nx (the padding of the last block) are never written: the buffers must be
 // zero-initialised once by the caller.
-template <typename T>
-struct SbSlabPlan {
-  int nzl, kxl, zl_shift;
-  long long blk;       // elements of one destination / source block
-  SbLines lr, lbuf, lz;  // R lines along y, B lines along y, B lines along z
-};
-template <typename T>
-static SbSlabPlan<T> slab_plan(const sb200_poisson* p, const SbFftState<T>* st, int ncomp) {
-  SbSlabPlan<T> s;
-  const int P_ = p->nranks, nz = p->nz, ny = p->ny;
-  s.nzl = nz / P_;
-  s.kxl = st->kxl;
-  s.zl_shift = 0;
-  while ((1 << s.zl_shift) < s.nzl) ++s.zl_shift;
-  const long long kxl = s.kxl;
-  s.blk = (long long)ncomp * s.nzl * ny * kxl;
-  // R[zb][c][zl][y][kx]: lines (kx, z, c), points along y
-  s.lr = SbLines{s.kxl, nz, ncomp, (long long)ny * kxl, (long long)s.nzl * ny * kxl, kxl};
-  s.lr.o1_shift = s.zl_shift;
-  s.lr.s1_hi = s.blk;
-  // B[c][z][ky][kx]: lines (kx, z, c) along ky, and lines (kx, ky, c) along z
-  s.lbuf = SbLines{s.kxl, nz, ncomp, 2LL * ny * kxl, (long long)nz * 2 * ny * kxl, kxl};
-  s.lz = SbLines{s.kxl, 2 * ny, ncomp, kxl, (long long)nz * 2 * ny * kxl, 2LL * ny * kxl};
-  return s;
-}
-
-template <typename T>
-static int slab_forward_t(sb200_poisson* p, const void* rhs, int ncomp, void* send, void* stream) {
-  auto* st = (SbFftState<T>*)p->backend_state;
-  const int nzl = p->nz / p->nranks, ny = p->ny, nx = p->nx, gs = p->gs;
-  const long long my = ny + 2 * gs, mx = nx + 2 * gs, vol = (nzl + 2LL * gs) * my * mx;
-  const SbSlabPlan<T> sp = slab_plan<T>(p, st, ncomp);
-  FieldRows<T> src{(T*)rhs, ny, gs, 3, my, mx, vol};
-  return launch_x_r2c<T, FieldRows<T>, true>(st->px, ny, nzl, ncomp, src, (C2<T>*)send, 0, st->twx, st->wpost,
-                                             stream, sb_row_blocks(sp.kxl, sp.blk));
-}
-template <typename T>
-static int slab_spectral_t(sb200_poisson* p, void* recv, int ncomp, void* stream) {
-  auto* st = (SbFftState<T>*)p->backend_state;
-  const SbSlabPlan<T> sp = slab_plan<T>(p, st, ncomp);
-  SbGreensTable<T> none{nullptr, 0, 0};
-  int e;
-  if (st->zconv) {
-    // tile-contiguous B (see fft_solve_t): Bt[c][kx group][ky][z][8]; the padding lines of the last group
-    // stay zero
-    const long long NKY = 2LL * p->ny, tile = (long long)p->nz * 8;
-    SbLines lb{sp.kxl, p->nz, ncomp, 8, (long long)st->ng * NKY * tile, tile};
-    lb.gsh = 3;
-    lb.s_grp = NKY * tile;
-    lb.rot = 7;
-    if ((e = launch_strided<T, 0>(st->py, (const C2<T>*)recv, sp.lr, st->B, lb, st->twy, none, stream))) return e;
-    if ((e = launch_zconv<T>(st->pz.log2n, st->B, ncomp, st->ng, (int)NKY, st->twz, st->G2, 2 * p->ny, st->tile_counter,
-                             stream)))
-      return e;
-    return launch_strided<T, 2>(st->py, st->B, lb, (C2<T>*)recv, sp.lr, st->twy, none, stream);
-  }
-  if ((e = launch_strided<T, 0>(st->py, (const C2<T>*)recv, sp.lr, st->B, sp.lbuf, st->twy, none, stream))) return e;
-  SbGreensTable<T> gt{st->G, (long long)(p->ny + 1) * st->P, st->P, 2 * p->ny, 0};
-  gt.g2 = st->G2;
-  gt.kx0 = p->rank * sp.kxl;
-  gt.kx_last = (int)st->P - 1;
-  if ((e = launch_strided<T, 1>(st->pz, st->B, sp.lz, st->B, sp.lz, st->twz, gt, stream))) return e;
-  return launch_strided<T, 2>(st->py, st->B, sp.lbuf, (C2<T>*)recv, sp.lr, st->twy, none, stream);
-}
-template <typename T>
-static int slab_backward_t(sb200_poisson* p, void* solution, int ncomp, const void* send, void* stream) {
-  auto* st = (SbFftState<T>*)p->backend_state;
-  const int nzl = p->nz / p->nranks, ny = p->ny, nx = p->nx, gs = p->gs;
-  const long long my = ny + 2 * gs, mx = nx + 2 * gs, vol = (nzl + 2LL * gs) * my * mx;
-  const SbSlabPlan<T> sp = slab_plan<T>(p, st, ncomp);
-  FieldRows<T> dst{(T*)solution, ny, gs, 3, my, mx, vol};
-  return launch_x_c2r<T>(st->px, ny, nzl, ncomp, (const C2<T>*)send, 0, dst, (const C2<T>*)st->twx,
-                         (const C2<T>*)st->wpost, stream, sb_row_blocks(sp.kxl, sp.blk));
-}
-
 static int slab_check(const sb200_poisson* p, int ncomp) {
   SB_REQUIRE(p && p->backend == 1 && p->nranks > 1 && p->backend_state,
              "poisson slab entry points need a distributed handle of the fft backend");
@@ -1283,16 +1250,16 @@ extern "C" int64_t sb200_poisson_slab_buffer_bytes(const sb200_poisson_t* p, int
 extern "C" int sb200_poisson_slab_forward(sb200_poisson_t* p, const void* rhs, int ncomp, void* send_buf,
                                           void* stream) {
   if (int e = slab_check(p, ncomp)) return e;
-  SB_DISPATCH_DTYPE(p->dtype, return slab_forward_t<T>(p, rhs, ncomp, send_buf, stream));
+  SB_DISPATCH_DTYPE(p->dtype, return fft_x_forward_t<T>(p, rhs, ncomp, (C2<T>*)send_buf, stream));
 }
 extern "C" int sb200_poisson_slab_spectral(sb200_poisson_t* p, void* recv_buf, int ncomp, void* stream) {
   if (int e = slab_check(p, ncomp)) return e;
-  SB_DISPATCH_DTYPE(p->dtype, return slab_spectral_t<T>(p, recv_buf, ncomp, stream));
+  SB_DISPATCH_DTYPE(p->dtype, return fft_spectral_t<T>(p, (C2<T>*)recv_buf, ncomp, stream));
 }
 extern "C" int sb200_poisson_slab_backward(sb200_poisson_t* p, void* solution, int ncomp, const void* send_buf,
                                            void* stream) {
   if (int e = slab_check(p, ncomp)) return e;
-  SB_DISPATCH_DTYPE(p->dtype, return slab_backward_t<T>(p, solution, ncomp, send_buf, stream));
+  SB_DISPATCH_DTYPE(p->dtype, return fft_x_backward_t<T>(p, solution, ncomp, (const C2<T>*)send_buf, stream));
 }
 int sb_poisson_fft_destroy(sb200_poisson* p) {
   if (p->dtype == SB200_F32) fft_destroy_t<float>(p); else fft_destroy_t<double>(p);

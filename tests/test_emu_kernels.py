@@ -381,9 +381,12 @@ def _slab_solve_emulated(lib, real_t, n, nranks, rhs, gs, ncomp):
 @pytest.mark.parametrize("real_t,n,nranks", [
     (np.float64, (16, 8, 32), 2), (np.float64, (32, 16, 16), 4), (np.float32, (128, 8, 16), 2),
     (np.float32, (16, 128, 32), 2), (np.float32, (32, 8, 64), 8),
+    # 2 nz = 512 / 1024: the tile-layout z kernel (sb_fft_zconvw_kernel)
+    (np.float32, (256, 8, 16), 2), (np.float32, (512, 8, 16), 4),
 ], ids=lambda v: str(v) if not isinstance(v, type) else v.__name__)
 def test_slab_decomposed_poisson_pipeline(real_t, n, nranks):
-    """The distributed (z-slab) solve, all ranks emulated in one process, against the scipy oracle."""
+    """The distributed (z-slab) solve, all ranks emulated in one process, against the scipy oracle and,
+    bit for bit, against the single-domain solve (the same three stages on a one-rank layout)."""
     from emu_util import emu
     from oracle.poisson import UnboundedPoissonSolverOracle3D
 
@@ -393,6 +396,12 @@ def test_slab_decomposed_poisson_pipeline(real_t, n, nranks):
     shape = tuple(v + 2 * gs for v in n)
     rhs = rng.uniform(size=(ncomp,) + shape).astype(real_t)
     out = _slab_solve_emulated(lib, real_t, n, nranks, rhs, gs, ncomp)
+    h = ctypes.c_void_p()
+    _lib.check(lib, lib.sb200_poisson_create(ctypes.byref(h), 3, _lib.dtype_code(real_t), n[0], n[1], n[2],
+                                             gs, 1.0, 0, 1, 1, None))
+    single = np.full_like(rhs, 7.0)
+    _lib.check(lib, lib.sb200_poisson_solve(h, ptr(single), ptr(rhs), ncomp, None))
+    lib.sb200_poisson_destroy(h)
     oracle = UnboundedPoissonSolverOracle3D(*n, x_range=1.0, real_t=real_t)
     ref = np.zeros_like(rhs)
     for c in range(ncomp):
@@ -404,6 +413,7 @@ def test_slab_decomposed_poisson_pipeline(real_t, n, nranks):
         got = out[r][:, gs:-gs, gs:-gs, gs:-gs]
         want = ref[:, r * nzl + gs:r * nzl + gs + nzl, gs:-gs, gs:-gs]
         assert np.abs(got - want).max() / scale < tol, (r, np.abs(got - want).max() / scale)
+        assert np.array_equal(got, single[:, r * nzl + gs:r * nzl + gs + nzl, gs:-gs, gs:-gs]), r
         assert np.all(out[r][:, 0] == 7.0) and np.all(out[r][:, :, :, -1] == 7.0)  # ghosts untouched
 
 

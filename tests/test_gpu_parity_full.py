@@ -433,13 +433,12 @@ def test_slab_poisson_with_virtual_ranks_on_one_gpu(cuda, n, real_t, nranks):
         oracle.vector_field_solve(want, rhs.cpu().numpy(), gs)
         inner = (slice(None),) + (slice(gs, -gs),) * 3
         assert _rel(ref.cpu().numpy()[inner], want[inner]) <= TOL[real_t]
+    # the single-domain solve runs the same three stages on a one-rank layout: bit for bit the same result
     nzl = n[0] // nranks
-    scale = ref.abs().max().item()
-    tol = 2e-6 if real_t == np.float32 else 1e-12
     for r in range(nranks):
         got = outs[r][:, gs:-gs, gs:-gs, gs:-gs]
         want = ref[:, r * nzl + gs:r * nzl + gs + nzl, gs:-gs, gs:-gs]
-        assert (got - want).abs().max().item() / scale <= tol, r
+        assert torch.equal(got, want), (r, (got - want).abs().max().item() / ref.abs().max().item())
         assert torch.all(outs[r][:, 0] == 7.0) and torch.all(outs[r][:, :, :, -1] == 7.0)  # ghosts untouched
 
 
