@@ -158,14 +158,11 @@ class _UnboundedPoissonSolver:
 
         lib, h = self.lib, self._handle
         if not self._slab_bufs:
-            import os
-
             from ...utils.peer import PeerExchange
 
             nfloat = int(lib.sb200_poisson_slab_buffer_bytes(h, 1)) // 4
             # per component a (send, recv) pair, visible to the other ranks through CUDA IPC
-            self._peer = PeerExchange(6, nfloat, self.device, self.mpi_construct.rank, self.mpi_construct.size,
-                                      use_peer_copies=os.environ.get("SB200_NO_PEER_COPIES") is None)
+            self._peer = PeerExchange(6, nfloat, self.device, self.mpi_construct.rank, self.mpi_construct.size)
             self.exchange_mode = self._peer.mode
             self._slab_bufs = [(self._peer.local[2 * c], self._peer.local[2 * c + 1]) for c in range(3)]
             # high priority: the NCCL kernels must get SMs while a transform kernel still has blocks queued

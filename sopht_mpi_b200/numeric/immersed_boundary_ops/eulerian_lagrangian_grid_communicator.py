@@ -10,10 +10,8 @@ import ctypes
 
 import numpy as np
 import torch
-import torch.distributed as dist
 
 from ... import _lib
-from ...utils.comm import MPI
 from ...utils.device import Staged, current_stream_ptr, dptr, torch_dtype
 
 
@@ -43,44 +41,22 @@ class MPIGhostSumCommunicator:
         stream = current_stream_ptr(mc.device)
         if mc.size > 1:
             comps = [f] if ncomp == 1 else [f[c] for c in range(ncomp)]
-            prev, nxt = int(mc.previous_grid_along[0]), int(mc.next_grid_along[0])
             key = (ncomp, f.dtype)
             if key not in self._bufs:
                 shape = (ncomp, gs) + tuple(comps[0].shape[1:])
                 self._bufs[key] = (torch.zeros(shape, dtype=f.dtype, device=f.device),
                                    torch.zeros(shape, dtype=f.dtype, device=f.device))
-            from_prev, from_next = self._bufs[key]
+            recv_prev, recv_next = self._bufs[key]
             from ...utils.peer import peer_halo
 
             up, down = [t[-gs:] for t in comps], [t[:gs] for t in comps]
-            halo = peer_halo(mc, up[0].numel() * up[0].element_size()) if f.is_cuda else None
-            if halo is not None and halo.usable(up, down):
-                # ghost slabs straight into the neighbours' mailboxes; the add kernel reads them there
-                ticket = halo.send(up, down)
-                p_prev, p_next = halo.wait(ticket, ncomp, ncomp)
-                _lib.check(self.lib, self.lib.sb200_ghost_sum_add_z(
-                    ctypes.byref(self.grid), dptr(f), ncomp,
-                    ctypes.c_void_p(p_prev) if prev != MPI.PROC_NULL else None,
-                    ctypes.c_void_p(p_next) if nxt != MPI.PROC_NULL else None, stream))
-                _lib.check(self.lib, self.lib.sb200_clear_ghost_cells(ctypes.byref(self.grid), dptr(f), ncomp,
-                                                                     stream))
-                st.finish()
-                return
-            ops = []
-            for c, t in enumerate(comps):
-                if nxt != MPI.PROC_NULL:
-                    ops.append(dist.P2POp(dist.isend, t[-gs:], nxt, tag=2 * c))
-                if prev != MPI.PROC_NULL:
-                    ops.append(dist.P2POp(dist.irecv, from_prev[c], prev, tag=2 * c))
-                    ops.append(dist.P2POp(dist.isend, t[:gs], prev, tag=2 * c + 1))
-                if nxt != MPI.PROC_NULL:
-                    ops.append(dist.P2POp(dist.irecv, from_next[c], nxt, tag=2 * c + 1))
-            for req in dist.batch_isend_irecv(ops) if ops else []:
-                req.wait()
+            halo = peer_halo(mc, up[0].numel() * up[0].element_size())
+            # the add kernel reads the received slabs where they are (mailbox or receive buffer)
+            from_prev, from_next = halo.finish(halo.start(up, down, list(recv_prev), list(recv_next)))
             _lib.check(self.lib, self.lib.sb200_ghost_sum_add_z(
                 ctypes.byref(self.grid), dptr(f), ncomp,
-                dptr(from_prev) if prev != MPI.PROC_NULL else None,
-                dptr(from_next) if nxt != MPI.PROC_NULL else None, stream))
+                ctypes.c_void_p(from_prev[0]) if from_prev else None,
+                ctypes.c_void_p(from_next[0]) if from_next else None, stream))
         _lib.check(self.lib, self.lib.sb200_clear_ghost_cells(ctypes.byref(self.grid), dptr(f), ncomp,
                                                              stream))
         st.finish()

@@ -249,9 +249,7 @@ class MPIGhostCommunicator:
         self.mpi_construct = mpi_construct
         self.full_exchange = full_exchange
         self.grid_coord = np.array(mpi_construct.grid.coords)
-        self.comm_requests = []
-        self._peer_pending = []  # (halo, ticket, fields) of exchanges that went through peer memory
-        self._recv_staging = []
+        self.comm_requests = []  # (neighbour exchange, its pending exchange, fields) per started exchange
         # fields whose ghost planes are known to be current: (data_ptr, host-write version) of the last
         # exchange; the owner of a field drops the entry when a kernel rewrites it (``mark_stale``)
         self._fresh = {}
@@ -269,54 +267,25 @@ class MPIGhostCommunicator:
             t[tuple(lo)] = t[tuple(src_lo)].clone()
             t[tuple(hi)] = t[tuple(src_hi)].clone()
 
-    def _plane_ops(self, t):
-        """P2P operations of one scalar field: "up" messages go to the next slab, "down" messages
-        to the previous one; the posting order keeps both directions apart even when prev == next."""
-        mc = self.mpi_construct
-        gs = self.ghost_size
-        prev, nxt = int(mc.previous_grid_along[0]), int(mc.next_grid_along[0])
-        ops = []
-        if nxt != MPI.PROC_NULL:
-            ops.append(dist.P2POp(dist.isend, t[-2 * gs:-gs], nxt, tag=0))
-        if prev != MPI.PROC_NULL:
-            ops.append(dist.P2POp(dist.irecv, t[:gs], prev, tag=0))
-            ops.append(dist.P2POp(dist.isend, t[gs:2 * gs], prev, tag=1))
-        if nxt != MPI.PROC_NULL:
-            ops.append(dist.P2POp(dist.irecv, t[-gs:], nxt, tag=1))
-        return ops
-
     def _exchange_init(self, fields):
         mc = self.mpi_construct
         gs = self.ghost_size
-        ops = []
-        if mc.size > 1 and fields and all(t.is_cuda for t in fields):
-            # boundary planes straight into the neighbours' mailboxes (utils/peer.py:PeerHalo)
-            from .peer import peer_halo
-
+        if mc.periodic_domain:
+            for t in fields:
+                self._wrap_local_axes(t)
+        if mc.size == 1:
             if mc.periodic_domain:
                 for t in fields:
-                    self._wrap_local_axes(t)
-            up, down = [t[-2 * gs:-gs] for t in fields], [t[gs:2 * gs] for t in fields]
-            halo = peer_halo(mc, up[0].numel() * up[0].element_size())
-            if halo is not None and halo.usable(up, down):
-                self._peer_pending.append((halo, halo.send(up, down), list(fields)))
-                return
-            for t in fields:
-                ops += self._plane_ops(t)
-            if ops:
-                self.comm_requests += dist.batch_isend_irecv(ops)
-            return
-        for t in fields:
-            if mc.periodic_domain:
-                self._wrap_local_axes(t)
-            if mc.size == 1:
-                if mc.periodic_domain:
                     t[:gs] = t[-2 * gs:-gs].clone()
                     t[-gs:] = t[gs:2 * gs].clone()
-                continue
-            ops += self._plane_ops(t)
-        if ops:  # one NCCL group for all planes of all components
-            self.comm_requests += dist.batch_isend_irecv(ops)
+            return
+        from .peer import peer_halo
+
+        # boundary planes to the neighbours (their mailboxes, or messages straight into the ghost planes)
+        up, down = [t[-2 * gs:-gs] for t in fields], [t[gs:2 * gs] for t in fields]
+        halo = peer_halo(mc, up[0].numel() * up[0].element_size())
+        pending = halo.start(up, down, [t[:gs] for t in fields], [t[-gs:] for t in fields])
+        self.comm_requests.append((halo, pending, list(fields)))
 
     def exchange_scalar_field_init(self, local_field):
         t, _ = _tensor_of(local_field)
@@ -333,23 +302,17 @@ class MPIGhostCommunicator:
             self.mark_fresh(local_vector_field)
 
     def exchange_finalise(self):
-        for req in self.comm_requests:
-            req.wait()
-        self.comm_requests = []
         gs = self.ghost_size
-        for halo, ticket, fields in self._peer_pending:
-            n, nbytes = len(fields), ticket[4] or fields[0][:gs].numel() * fields[0].element_size()
-            from_prev, from_next = halo.wait(ticket, n, n)
+        for halo, pending, fields in self.comm_requests:
+            from_prev, from_next = halo.finish(pending)
             dst, src = [], []
             for c, t in enumerate(fields):
-                if halo.prev is not None:
-                    dst.append(t[:gs].data_ptr())
-                    src.append(from_prev + c * nbytes)
-                if halo.next is not None:
-                    dst.append(t[-gs:].data_ptr())
-                    src.append(from_next + c * nbytes)
-            halo.copy_blocks(dst, src, nbytes)
-        self._peer_pending = []
+                for received, ghost in ((from_prev, t[:gs]), (from_next, t[-gs:])):
+                    if received and received[c] != ghost.data_ptr():  # (not yet in the ghost plane)
+                        dst.append(ghost.data_ptr())
+                        src.append(received[c])
+            halo.copy_blocks(dst, src, fields[0][:gs].numel() * fields[0].element_size())
+        self.comm_requests = []
 
     # ---- ghost freshness (B200 build): lets the simulator skip an exchange of a field whose ghost
     # planes were filled since it was last written (the interactor exchanges the velocity right before

@@ -106,7 +106,7 @@ def check_block_exchange():
     from sopht_mpi_b200.utils.peer import PeerExchange
 
     rank, size = dist.get_rank(), dist.get_world_size()
-    ex = PeerExchange(2, 6 * size, torch.device("cpu"), rank, size, use_peer_copies=False)
+    ex = PeerExchange(2, 6 * size, torch.device("cpu"), rank, size)
     assert ex.mode == "nccl all-to-all"
     ex.local[0].copy_(torch.arange(6 * size, dtype=torch.float32) + 100 * rank)
     try:

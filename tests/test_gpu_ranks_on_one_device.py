@@ -49,7 +49,6 @@ def test_peer_halo_and_ghost_sum_with_three_processes_on_one_gpu():
 def test_slab_decomposition_with_all_ranks_on_one_gpu(size):
     """tests/dist_gpu_worker.py (slab Poisson solve over the peer-memory all-to-all, halo exchange + fused
     steps, IB ownership / forces / ghost sum against the single-domain oracle) with every rank on cuda:0"""
-    # (the push-kernel transport: peer copies between two contexts of ONE device are not what the
-    # copy-engine transport is for; tests/test_gpu_multi.py runs that one on 2 and 4 real GPUs)
-    _run_ranks_on_one_gpu("dist_gpu_worker.py", size, "DIST_GPU_WORKER_OK",
-                          {"SB200_TEST_SINGLE_DEVICE": "1", "SB200_EXCHANGE": "push"})
+    # (ranks that share a device take the push-kernel transport; tests/test_gpu_multi.py runs the copy-engine
+    # transport on 2 and 4 real GPUs)
+    _run_ranks_on_one_gpu("dist_gpu_worker.py", size, "DIST_GPU_WORKER_OK", {"SB200_TEST_SINGLE_DEVICE": "1"})

@@ -551,7 +551,7 @@ def test_bench_step_with_ranks_on_one_gpu(name, nranks, tmp_path, record_propert
     try:
         _bench_step_single_gpu_runs(name, tmp_path)
         _run_ranks_on_one_gpu("dist_bench_step_worker.py", nranks, "DIST_BENCH_STEP_WORKER_OK",
-                              {"SB200_TEST_SINGLE_DEVICE": "1", "SB200_EXCHANGE": "push", "SB200_PEER_WAIT_S": "300",
+                              {"SB200_TEST_SINGLE_DEVICE": "1", "SB200_PEER_WAIT_S": "300",
                                "SB200_BENCH_STEP_WORKLOAD": name, "SB200_BENCH_STEP_DIR": str(tmp_path)})
         _check_bench_step(name, nranks, tmp_path, record_property)
     finally:

@@ -3,7 +3,7 @@
 cd /root/repo
 port=$((20000 + RANDOM % 20000))
 for r in $(seq 0 $(($1 - 1))); do
-  RANK=$r WORLD_SIZE=$1 LOCAL_RANK=0 MASTER_ADDR=127.0.0.1 MASTER_PORT=$port SB200_TEST_SINGLE_DEVICE=1 SB200_EXCHANGE=push SB200_PEER_WAIT_S=${SB200_PEER_WAIT_S:-60} \
+  RANK=$r WORLD_SIZE=$1 LOCAL_RANK=0 MASTER_ADDR=127.0.0.1 MASTER_PORT=$port SB200_TEST_SINGLE_DEVICE=1 SB200_PEER_WAIT_S=${SB200_PEER_WAIT_S:-60} \
     python tests/dist_gpu_worker.py > gpurun_out/sd_$r.log 2>&1 &
 done
 wait
