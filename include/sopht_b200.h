@@ -182,13 +182,16 @@ int sb200_poisson_destroy(sb200_poisson_t* p);
 /* single-rank solve of `ncomp` components: psi interior <- solve(rhs interior) */
 int sb200_poisson_solve(sb200_poisson_t* p, void* solution, const void* rhs, int ncomp, void* stream);
 int64_t sb200_poisson_workspace_bytes(const sb200_poisson_t* p);
-/* z-slab decomposition (nranks = 2, 4 or 8; backend 1): mpi4py-fft's distributed transform
+/* z-slab decomposition.  Served by distributed handles (nranks > 1, 3D) of either backend: backend 1
+ * on 2, 4 or 8 ranks for power-of-two grids, backend 0 (cuFFT) on any rank count that divides nz, for
+ * any grid size.  Both use the same buffers and layout.  mpi4py-fft's distributed transform
  * (poisson_solver_3d/fft_mpi_3d.py:27-48) and MPIDomainDoublingCommunicator3D
  * (UnboundedPoissonSolverMPI3D.py:190-382) become
  *   slab_forward  (x r2c of the local planes -> send_buf, blocked by destination rank: each rank
  *                  receives ceil((nx+1)/nranks) kx bins, rounded up to a multiple of 4, of every plane)
  *   all-to-all  send_buf -> recv_buf                       (caller: NCCL)
- *   slab_spectral (y forward, fused z forward x Green x z inverse, y inverse; result back in recv_buf)
+ *   slab_spectral (y and z forward on the zero-padded doubled plane x Green x inverse, cropped;
+ *                  result back in recv_buf)
  *   all-to-all  recv_buf -> send_buf
  *   slab_backward (x c2r of the local planes -> solution interior)
  * The transposes act on the x-pass output, the smallest array of the pipeline (2 reals per cell

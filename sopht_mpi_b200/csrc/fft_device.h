@@ -14,6 +14,10 @@ struct alignas(2 * sizeof(T)) C2 {
   T x, y;
 };
 
+// device table W[k] = exp(-2 pi i k / denom), k < count (poisson_fft.cu); nullptr when the allocation fails
+template <typename T>
+C2<T>* make_twiddles(int n, int count, double denom, void* stream);
+
 template <typename T>
 SB_HD C2<T> cmul(C2<T> a, C2<T> b) {
   return C2<T>{a.x * b.x - a.y * b.y, a.x * b.y + a.y * b.x};

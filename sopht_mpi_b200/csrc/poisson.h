@@ -64,10 +64,46 @@ void sb_poisson_free_greens_lines(void* lines_dev);
 // (UnboundedPoissonSolverMPI3D.py:82-114 / UnboundedPoissonSolverMPI2D.py:73-101).
 int sb_poisson_fill_greens(const sb200_poisson* p, void* dst, void* stream);
 
+// The exchange format of the z-slab solve, shared by both backends.
+// Rows of kx bins either contiguous (pitch elements per row) or, for the x-slab transpose of the
+// distributed solve, split into blocks of kxl bins: bin k of row `line` lives at
+//   (k / kxl) * blk + line * kxl + k % kxl        (one block per destination / source rank)
+// kx bins per rank of the x-slab decomposition: ceil((nx + 1) / nranks) rounded up to a multiple of
+// 4 so that every row of a block starts on a 32-byte sector
+static inline int sb_slab_kxl(int nx, int nranks) { return ((nx + 1 + nranks - 1) / nranks + 3) & ~3; }
+
+struct SbRowBlocks {
+  int kxl = 0;          // 0: contiguous rows
+  unsigned magic = 0;   // ceil(2^32 / kxl): k / kxl == umulhi(k, magic) for k * kxl < 2^32
+  long long dblk = 0;   // block stride minus kxl
+  // element offset of bin k relative to the start of its row in block 0
+  SB_D long long rel(int k) const {
+#ifdef SB200_EMU
+    const int b = k / kxl;
+#else
+    const int b = (int)__umulhi((unsigned)k, magic);
+#endif
+    return (long long)b * dblk + k;
+  }
+  SB_D long long row(long long line, long long pitch) const { return line * (kxl ? (long long)kxl : pitch); }
+};
+static inline SbRowBlocks sb_row_blocks(int kxl, long long blk) {
+  SbRowBlocks rb;
+  rb.kxl = kxl;
+  rb.magic = kxl ? (unsigned)((0x100000000ULL + (unsigned long long)kxl - 1) / (unsigned long long)kxl) : 0;
+  rb.dblk = blk - kxl;
+  return rb;
+}
+
 int sb_poisson_cufft_create(sb200_poisson* p, void* stream);
 int sb_poisson_cufft_destroy(sb200_poisson* p);
 int sb_poisson_cufft_solve(sb200_poisson* p, void* solution, const void* rhs, int ncomp, void* stream);
 int64_t sb_poisson_cufft_bytes(const sb200_poisson* p);
+// z-slab stages of a distributed cuFFT handle (any grid size, any rank count that divides nz)
+int sb_poisson_cufft_slab_forward(sb200_poisson* p, const void* rhs, int ncomp, void* send_buf, void* stream);
+int sb_poisson_cufft_slab_spectral(sb200_poisson* p, void* recv_buf, int ncomp, void* stream);
+int sb_poisson_cufft_slab_backward(sb200_poisson* p, void* solution, int ncomp, const void* send_buf,
+                                   void* stream);
 
 int sb_poisson_fft_create(sb200_poisson* p, void* stream);
 int sb_poisson_fft_destroy(sb200_poisson* p);

@@ -80,36 +80,6 @@ struct GreensRows {
   SB_D C2<T> load(int, int z, int y, int m) const { return C2<T>{g(z, y, 2 * m), g(z, y, 2 * m + 1)}; }
 };
 
-// Rows of kx bins either contiguous (pitch elements per row) or, for the x-slab transpose of the
-// distributed solve, split into blocks of kxl bins: bin k of row `line` lives at
-//   (k / kxl) * blk + line * kxl + k % kxl        (one block per destination / source rank)
-// kx bins per rank of the x-slab decomposition: ceil((nx + 1) / nranks) rounded up to a multiple of
-// 4 so that every row of a block starts on a 32-byte sector
-static inline int sb_slab_kxl(int nx, int nranks) { return ((nx + 1 + nranks - 1) / nranks + 3) & ~3; }
-
-struct SbRowBlocks {
-  int kxl = 0;          // 0: contiguous rows
-  unsigned magic = 0;   // ceil(2^32 / kxl): k / kxl == umulhi(k, magic) for k * kxl < 2^32
-  long long dblk = 0;   // block stride minus kxl
-  // element offset of bin k relative to the start of its row in block 0
-  SB_D long long rel(int k) const {
-#ifdef SB200_EMU
-    const int b = k / kxl;
-#else
-    const int b = (int)__umulhi((unsigned)k, magic);
-#endif
-    return (long long)b * dblk + k;
-  }
-  SB_D long long row(long long line, long long pitch) const { return line * (kxl ? (long long)kxl : pitch); }
-};
-static inline SbRowBlocks sb_row_blocks(int kxl, long long blk) {
-  SbRowBlocks rb;
-  rb.kxl = kxl;
-  rb.magic = kxl ? (unsigned)((0x100000000ULL + (unsigned long long)kxl - 1) / (unsigned long long)kxl) : 0;
-  rb.dblk = blk - kxl;
-  return rb;
-}
-
 // ------------------------------------------------------------------ x pass: r2c
 // Real rows of length 2N (second half zero when PRUNED) -> N+1 bins through ONE complex FFT
 // of length N on z[m] = x[2m] + i x[2m+1]:
@@ -793,7 +763,7 @@ struct SbFftState {
 };
 
 template <typename T>
-static C2<T>* make_twiddles(int n, int count, double denom, void* stream) {
+C2<T>* make_twiddles(int n, int count, double denom, void* stream) {
   // W[k] = exp(-2 pi i k / denom), k < count
   std::vector<C2<T>> h(count);
   for (int k = 0; k < count; ++k) {
@@ -807,6 +777,8 @@ static C2<T>* make_twiddles(int n, int count, double denom, void* stream) {
   (void)n;
   return d;
 }
+template C2<float>* make_twiddles<float>(int, int, double, void*);
+template C2<double>* make_twiddles<double>(int, int, double, void*);
 
 static int lines_per_block_for(int threads_per_line, size_t elem, bool strided) {
   int lb = strided ? (elem == 4 ? 8 : 4) : 1;  // >= 64 B contiguous per point for strided passes
@@ -1233,11 +1205,13 @@ int sb_poisson_fft_create(sb200_poisson* p, void* stream) {
 //             kx0 + kx_in), y inverse B -> R (same blocked-by-z layout)
 //   all-to-all back, backward: x c2r of the local planes from S.
 // The three stages are the ones of the single-GPU solve (fft_solve_t) on the caller's buffers.
+// A distributed handle of the cuFFT backend (any grid size, any rank count that divides nz) runs the same
+// three stages on the same buffers (poisson_cufft.cu).
 // Bins beyond nx (the padding of the last block) are never written: the buffers must be
 // zero-initialised once by the caller.
 static int slab_check(const sb200_poisson* p, int ncomp) {
-  SB_REQUIRE(p && p->backend == 1 && p->nranks > 1 && p->backend_state,
-             "poisson slab entry points need a distributed handle of the fft backend");
+  SB_REQUIRE(p && (p->backend == 0 || p->backend == 1) && p->nranks > 1 && p->backend_state,
+             "poisson slab entry points need a distributed handle");
   SB_REQUIRE(ncomp >= 1 && ncomp <= 3, "poisson slab: ncomp must be 1..3");
   return 0;
 }
@@ -1250,15 +1224,18 @@ extern "C" int64_t sb200_poisson_slab_buffer_bytes(const sb200_poisson_t* p, int
 extern "C" int sb200_poisson_slab_forward(sb200_poisson_t* p, const void* rhs, int ncomp, void* send_buf,
                                           void* stream) {
   if (int e = slab_check(p, ncomp)) return e;
+  if (p->backend == 0) return sb_poisson_cufft_slab_forward(p, rhs, ncomp, send_buf, stream);
   SB_DISPATCH_DTYPE(p->dtype, return fft_x_forward_t<T>(p, rhs, ncomp, (C2<T>*)send_buf, stream));
 }
 extern "C" int sb200_poisson_slab_spectral(sb200_poisson_t* p, void* recv_buf, int ncomp, void* stream) {
   if (int e = slab_check(p, ncomp)) return e;
+  if (p->backend == 0) return sb_poisson_cufft_slab_spectral(p, recv_buf, ncomp, stream);
   SB_DISPATCH_DTYPE(p->dtype, return fft_spectral_t<T>(p, (C2<T>*)recv_buf, ncomp, stream));
 }
 extern "C" int sb200_poisson_slab_backward(sb200_poisson_t* p, void* solution, int ncomp, const void* send_buf,
                                            void* stream) {
   if (int e = slab_check(p, ncomp)) return e;
+  if (p->backend == 0) return sb_poisson_cufft_slab_backward(p, solution, ncomp, send_buf, stream);
   SB_DISPATCH_DTYPE(p->dtype, return fft_x_backward_t<T>(p, solution, ncomp, (const C2<T>*)send_buf, stream));
 }
 int sb_poisson_fft_destroy(sb200_poisson* p) {

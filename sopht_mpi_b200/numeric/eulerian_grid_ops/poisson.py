@@ -13,6 +13,15 @@ def _is_pow2(n):
     return n > 0 and (n & (n - 1)) == 0
 
 
+# Smallest 3D grid (cells) whose cuFFT solve runs on z-slabs when distributed; smaller grids stay replicated.
+# A tiny solve is bound by launches and latency, so the two exchanges per component of the slab pipeline
+# (six per vector solve) cost more than one all-gather there.  PROVISIONAL: the crossover has not been
+# measured on several GPUs.  2^18 cells (64^3) keeps the small grids the replicated path serves, e.g.
+# (6P, 20, 36) on up to 8 ranks (<= 34560 cells), replicated; DESIGN section 5 gives the reasoning and
+# tools/bench_slab_cufft.py is the measurement to set it from.
+_SLAB_CUFFT_MIN_CELLS = 1 << 18
+
+
 class _UnboundedPoissonSolver:
     def __init__(self, dim, grid_size, mpi_construct, ghost_size, x_range, real_t, backend):
         self.lib = _lib.load()
@@ -36,18 +45,20 @@ class _UnboundedPoissonSolver:
             small_enough = gs3[2] <= 4096 and gs3[1] <= 2048 and gs3[0] <= 2048
             backend = ("fft" if (pow2 and big_enough and small_enough
                                  and _fft_backend_available(self.lib)) else "cufft")
-        # Distributed solve.  The slab pipeline (transposes over NVLink, see _solve_slabs) covers 3D
-        # power-of-two grids on 2, 4 or 8 leading-axis slabs that are at least 2 ghost_size thick.
-        # Everything else the reference's mpi4py-fft path accepts (2D decompositions such as BASELINE
-        # configs[0]'s `-np 2` cylinder, other grid sizes, other rank counts) runs REPLICATED: the slab
-        # interiors are all-gathered over NCCL, every GPU solves the whole (then small or odd-sized)
-        # domain with the single-rank solver and keeps its own slab.
+        # Distributed solve.  The slab pipeline (transposes over NVLink, see _solve_slabs) covers 3D grids
+        # split into leading-axis slabs at least 2 ghost_size thick: power-of-two grids on 2, 4 or 8 ranks
+        # through the in-kernel transforms, every other grid through the cuFFT backend's z-slab mode on any
+        # rank count, once the grid reaches _SLAB_CUFFT_MIN_CELLS.  Everything else the reference's
+        # mpi4py-fft path accepts (2D decompositions such as BASELINE configs[0]'s `-np 2` cylinder, small
+        # grids) runs REPLICATED: the slab interiors are all-gathered over NCCL, every GPU solves the whole
+        # (then small) domain with the single-rank solver and keeps its own slab.
         self.replicated = False
         if mpi_construct.size > 1:
             size = mpi_construct.size
             lead = gs3[3 - dim]
-            slab_ok = (backend == "fft" and dim == 3 and size in (2, 4, 8) and lead % size == 0
-                       and lead // size >= 2 * ghost_size)
+            slab_ok = (dim == 3 and lead % size == 0 and lead // size >= 2 * ghost_size
+                       and ((backend == "fft" and size in (2, 4, 8))
+                            or (backend == "cufft" and gs3[0] * gs3[1] * gs3[2] >= _SLAB_CUFFT_MIN_CELLS)))
             if not slab_ok:
                 self.replicated = True
                 if backend == "fft" and not all(_is_pow2(int(g)) for g in grid_size):
