@@ -22,6 +22,7 @@ ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
 sys.path.insert(0, ROOT)
 
 import bench  # noqa: E402
+from harness import join_ranks, leave_ranks  # noqa: E402
 
 FIELDS = ("vorticity_field", "velocity_field", "stream_func_field")
 
@@ -158,32 +159,13 @@ def main():
             write_reference(name, path, torch.device("cuda", 0))
         print("DIST_BENCH_STEP_REFERENCE_OK")
         return
-    if os.environ.get("SB200_TEST_SINGLE_DEVICE"):
-        # every rank on cuda:0, gloo for the collectives (the peer-memory exchanges are the same CUDA IPC
-        # transports as on several GPUs)
-        torch.cuda.set_device(0)
-        dist.init_process_group(backend="gloo")
-    else:
-        from sopht_mpi_b200.utils.comm import init_process_group_if_needed
-
-        init_process_group_if_needed()
+    join_ranks()
     rank, size = dist.get_rank(), dist.get_world_size()
     device = torch.device("cuda", torch.cuda.current_device())
     sim, interactor = check_rank(name, path, device, rank, size, f"rank{rank}.json")
-    # release the CUDA-IPC mappings of the other ranks' exchange buffers before any rank exits (bench.py)
-    import gc
-
-    sim.unbounded_poisson_solver.close()
-    halo = getattr(sim.mpi_construct, "_peer_halo", None)
-    if halo is not None:
-        halo.close()
+    closables = (sim.unbounded_poisson_solver, getattr(sim.mpi_construct, "_peer_halo", None))
     del sim, interactor
-    gc.collect()
-    torch.cuda.ipc_collect()
-    dist.barrier()
-    if rank == 0:
-        print("DIST_BENCH_STEP_WORKER_OK")
-    dist.destroy_process_group()
+    leave_ranks("DIST_BENCH_STEP_WORKER_OK", *closables)
 
 
 if __name__ == "__main__":

@@ -11,6 +11,7 @@ import torch.distributed as dist
 ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
 sys.path.insert(0, ROOT)
 
+from harness import join_ranks, leave_ranks  # noqa: E402
 from oracle.poisson import UnboundedPoissonSolverOracle3D  # noqa: E402
 from oracle.simulator import FlowSimulatorOracle3D  # noqa: E402
 from oracle import ib as ib_oracle  # noqa: E402
@@ -25,11 +26,7 @@ def rel(a, b):
 
 
 def main():
-    if os.environ.get("SB200_TEST_SINGLE_DEVICE"):
-        # every rank on cuda:0, gloo for the collectives: the peer-memory transports (CUDA IPC between
-        # processes) are the same as on several GPUs, so a one-GPU box exercises the distributed path
-        torch.cuda.set_device(0)
-        dist.init_process_group(backend="gloo")
+    join_ranks()
     from sopht_mpi_b200.numeric.eulerian_grid_ops import UnboundedPoissonSolverMPI3D
     from sopht_mpi_b200.simulator import UnboundedFlowSimulator3D
     from sopht_mpi_b200.utils import MPIConstruct3D
@@ -158,14 +155,7 @@ def main():
     assert np.abs(got - want).max() / np.abs(f_glob).max() <= 1e-5
 
     check_replicated_solves(gs)
-
-    dist.barrier()
-    import gc
-
-    gc.collect()
-    if rank == 0:
-        print("DIST_GPU_WORKER_OK")
-    dist.destroy_process_group()
+    leave_ranks("DIST_GPU_WORKER_OK")
 
 
 def check_replicated_solves(gs):

@@ -13,10 +13,11 @@ import torch.distributed as dist
 ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
 sys.path.insert(0, ROOT)
 
+from harness import join_ranks, leave_ranks  # noqa: E402
+
 
 def main():
-    torch.cuda.set_device(0)
-    dist.init_process_group(backend="gloo")
+    join_ranks()
     from sopht_mpi_b200.numeric.immersed_boundary_ops.eulerian_lagrangian_grid_communicator import (
         MPIGhostSumCommunicator)
     from sopht_mpi_b200.utils import MPIConstruct3D, MPIGhostCommunicator3D
@@ -91,9 +92,7 @@ def main():
             dist.barrier()
             mc._peer_halo.close()
             mc._peer_halo = None
-    if rank == 0:
-        print("DIST_HALO_WORKER_OK")
-    dist.destroy_process_group()
+    leave_ranks("DIST_HALO_WORKER_OK")
 
 
 if __name__ == "__main__":

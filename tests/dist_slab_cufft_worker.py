@@ -7,11 +7,11 @@ import sys
 
 import numpy as np
 import torch
-import torch.distributed as dist
 
 ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
 sys.path.insert(0, ROOT)
 
+from harness import join_ranks, leave_ranks  # noqa: E402
 from oracle.poisson import UnboundedPoissonSolverOracle3D  # noqa: E402
 from oracle.simulator import FlowSimulatorOracle3D  # noqa: E402
 
@@ -20,9 +20,7 @@ N = (48, 72, 80)
 
 
 def main():
-    if os.environ.get("SB200_TEST_SINGLE_DEVICE"):
-        torch.cuda.set_device(0)
-        dist.init_process_group(backend="gloo")
+    join_ranks()
     from sopht_mpi_b200.numeric.eulerian_grid_ops import UnboundedPoissonSolverMPI3D
     from sopht_mpi_b200.simulator import UnboundedFlowSimulator3D
     from sopht_mpi_b200.utils import MPIConstruct3D
@@ -88,14 +86,7 @@ def main():
             err = np.abs(got - want).max() / np.abs(getattr(ora, name)).max()
             assert err <= tol, (name, real_t, err)
         sim.unbounded_poisson_solver.close()
-
-    dist.barrier()
-    import gc
-
-    gc.collect()
-    if dist.get_rank() == 0:
-        print("DIST_SLAB_CUFFT_WORKER_OK")
-    dist.destroy_process_group()
+    leave_ranks("DIST_SLAB_CUFFT_WORKER_OK")
 
 
 if __name__ == "__main__":

@@ -9,6 +9,7 @@ import torch.distributed as dist
 ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
 sys.path.insert(0, ROOT)
 
+from harness import join_ranks, leave_ranks  # noqa: E402
 from oracle import ib as ib_oracle  # noqa: E402
 from sopht_mpi_b200.utils import (MPIConstruct2D, MPIConstruct3D, MPIFieldCommunicator3D,  # noqa: E402
                                   MPIGhostCommunicator2D, MPIGhostCommunicator3D,
@@ -121,12 +122,10 @@ def check_block_exchange():
 
 
 if __name__ == "__main__":
-    check_halo_3d(periodic=False)  # (the first MPIConstruct joins the process group)
+    join_ranks()
+    check_halo_3d(periodic=False)
     check_block_exchange()
     check_halo_3d(periodic=True)
     check_field_comm_and_lagrangian()
     check_halo_2d()
-    dist.barrier()
-    if dist.get_rank() == 0:
-        print("DIST_WORKER_OK")
-    dist.destroy_process_group()
+    leave_ranks("DIST_WORKER_OK")

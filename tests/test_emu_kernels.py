@@ -9,12 +9,18 @@ import os
 import numpy as np
 import pytest
 
-from emu_util import call, ptr
+from harness import _call, _Host, emu, slab_poisson_solve
 from ib_helpers import rank_address
 from oracle import stencils as st
 from sopht_mpi_b200 import _lib
 
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
+_HOST = _Host()
+ptr = _HOST.ptr
+
+
+def call(fn_name, *args):
+    _call(_HOST, fn_name, *args)
 
 
 def _rel(a, b):
@@ -320,7 +326,6 @@ def test_ib_kernels_against_reference_golden(path):
 def test_pruned_fft_poisson_pipeline_3d(real_t, n):
     """backend 1 (in-kernel pruned FFT pipeline): every Stockham plan shape up to n = 1024
     against the scipy.fft oracle (which is what the reference's FFT test pins to)."""
-    from emu_util import emu
     from oracle.poisson import UnboundedPoissonSolverOracle3D
 
     lib = emu()
@@ -343,41 +348,6 @@ def test_pruned_fft_poisson_pipeline_3d(real_t, n):
     assert np.all(sol[:, 0] == 7.0) and np.all(sol[:, :, :, -1] == 7.0)  # ghosts untouched
 
 
-def _slab_solve_emulated(lib, real_t, n, nranks, rhs, gs, ncomp):
-    """Run the z-slab entry points of `nranks` handles in this process; the two all-to-alls are
-    numpy block transposes (what NCCL's all_to_all_single does with equal splits)."""
-    nzl = n[0] // nranks
-    handles = []
-    for r in range(nranks):
-        h = ctypes.c_void_p()
-        _lib.check(lib, lib.sb200_poisson_create(ctypes.byref(h), 3, _lib.dtype_code(real_t), n[0], n[1], n[2],
-                                                 gs, 1.0, r, nranks, 1, None))
-        handles.append(h)
-    nbytes = int(lib.sb200_poisson_slab_buffer_bytes(handles[0], ncomp))
-    itemsize = np.dtype(real_t).itemsize
-    send = [np.zeros(nbytes // itemsize, real_t) for _ in range(nranks)]
-    recv = [np.zeros(nbytes // itemsize, real_t) for _ in range(nranks)]
-    local = [np.ascontiguousarray(rhs[:, r * nzl:r * nzl + nzl + 2 * gs]) for r in range(nranks)]
-    out = [np.full_like(a, 7.0) for a in local]
-
-    def all_to_all(dst, src):
-        blk = src[0].size // nranks
-        for r in range(nranks):
-            for q in range(nranks):
-                dst[r][q * blk:(q + 1) * blk] = src[q][r * blk:(r + 1) * blk]
-
-    for r in range(nranks):
-        _lib.check(lib, lib.sb200_poisson_slab_forward(handles[r], ptr(local[r]), ncomp, ptr(send[r]), None))
-    all_to_all(recv, send)
-    for r in range(nranks):
-        _lib.check(lib, lib.sb200_poisson_slab_spectral(handles[r], ptr(recv[r]), ncomp, None))
-    all_to_all(send, recv)
-    for r in range(nranks):
-        _lib.check(lib, lib.sb200_poisson_slab_backward(handles[r], ptr(out[r]), ncomp, ptr(send[r]), None))
-        lib.sb200_poisson_destroy(handles[r])
-    return out
-
-
 @pytest.mark.parametrize("real_t,n,nranks", [
     (np.float64, (16, 8, 32), 2), (np.float64, (32, 16, 16), 4), (np.float32, (128, 8, 16), 2),
     (np.float32, (16, 128, 32), 2), (np.float32, (32, 8, 64), 8),
@@ -387,7 +357,6 @@ def _slab_solve_emulated(lib, real_t, n, nranks, rhs, gs, ncomp):
 def test_slab_decomposed_poisson_pipeline(real_t, n, nranks):
     """The distributed (z-slab) solve, all ranks emulated in one process, against the scipy oracle and,
     bit for bit, against the single-domain solve (the same three stages on a one-rank layout)."""
-    from emu_util import emu
     from oracle.poisson import UnboundedPoissonSolverOracle3D
 
     lib = emu()
@@ -395,7 +364,7 @@ def test_slab_decomposed_poisson_pipeline(real_t, n, nranks):
     rng = np.random.default_rng(1)
     shape = tuple(v + 2 * gs for v in n)
     rhs = rng.uniform(size=(ncomp,) + shape).astype(real_t)
-    out = _slab_solve_emulated(lib, real_t, n, nranks, rhs, gs, ncomp)
+    out = slab_poisson_solve(_Host(), n, real_t, nranks, rhs, ncomp, backend=1)
     h = ctypes.c_void_p()
     _lib.check(lib, lib.sb200_poisson_create(ctypes.byref(h), 3, _lib.dtype_code(real_t), n[0], n[1], n[2],
                                              gs, 1.0, 0, 1, 1, None))
@@ -421,7 +390,6 @@ def test_slab_decomposed_poisson_pipeline(real_t, n, nranks):
 @pytest.mark.parametrize("real_t, n", [(np.float64, (16, 32)), (np.float32, (16, 32)), (np.float32, (256, 16))],
                          ids=["f64", "f32", "f32-ny256"])
 def test_pruned_fft_poisson_pipeline_2d(real_t, n):
-    from emu_util import emu
     from oracle.poisson import UnboundedPoissonSolverOracle2D
 
     lib = emu()
@@ -572,8 +540,6 @@ def test_sparse_forcing_update_and_flagged_reset(dim, sparse):
         f *= mask
     ref, got = w.copy(), w.copy()
     call("sb200_update_vorticity_from_velocity_forcing", ctypes.byref(g), ptr(ref), ptr(f), 0.37, None)
-    from emu_util import emu
-
     count = int(emu().sb200_tile_flag_count(ctypes.byref(g)))
     work = np.zeros(count, np.uint8)
     call("sb200_update_vorticity_from_sparse_forcing", ctypes.byref(g), ptr(got), ptr(f), 0.37, ptr(work), None)

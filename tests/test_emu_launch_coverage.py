@@ -21,11 +21,10 @@ import subprocess
 import numpy as np
 import pytest
 
-from emu_util import emu
+from harness import _call, _fused_reference, _Host, cuda, emu, slab_poisson_solve  # noqa: F401
 from oracle import stencils as st
 from oracle.poisson import UnboundedPoissonSolverOracle2D, UnboundedPoissonSolverOracle3D
 from sopht_mpi_b200 import _lib
-from test_emu_kernels import _slab_solve_emulated
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "..", "sopht_mpi_b200", "csrc")
@@ -38,65 +37,6 @@ def _rel(a, b):
 
 def _tol(real_t):
     return 1e-13 if real_t == f64 else 2e-6
-
-
-class _Host:
-    """Buffers of the emulation: numpy arrays on the host."""
-
-    lib = property(lambda self: emu())
-
-    def dev(self, a, offset=0):
-        """a copy of `a` that starts `offset` elements after a 256-byte boundary (numpy itself only promises
-        16 bytes, less than the 32 the double vector kernels need)"""
-        buf = np.empty(a.nbytes + offset * a.itemsize + 256, np.uint8)
-        start = -buf.ctypes.data % 256 + offset * a.itemsize
-        out = buf[start:start + a.nbytes].view(a.dtype).reshape(a.shape)
-        out[...] = a
-        return out
-
-    def ptr(self, a):
-        return None if a is None else ctypes.c_void_p(a.ctypes.data)
-
-    def host(self, a):
-        return np.array(a)
-
-
-class _Cuda:
-    """Buffers of the CUDA library: torch tensors on cuda:0."""
-
-    def __init__(self):
-        import torch
-
-        self.torch = torch
-        self.lib = _lib.load()
-
-    def dev(self, a, offset=0):
-        t = self.torch
-        buf = t.empty(a.size + offset, dtype=t.float64 if a.dtype == f64 else t.float32 if a.dtype == f32 else
-                      t.uint8, device="cuda")
-        out = buf[offset:].view(a.shape)
-        out.copy_(t.from_numpy(np.ascontiguousarray(a)))
-        return out
-
-    def ptr(self, a):
-        return None if a is None else ctypes.c_void_p(a.data_ptr())
-
-    def host(self, a):
-        self.torch.cuda.synchronize()
-        return a.cpu().numpy()
-
-
-def _call(be, name, *args):
-    _lib.check(be.lib, getattr(be.lib, name)(*args))
-
-
-@pytest.fixture(scope="module")
-def cuda():
-    import torch
-
-    if not torch.cuda.is_available():
-        pytest.skip("no CUDA device")
-    return _Cuda()
 
 
 def _case_id(v):
@@ -190,7 +130,7 @@ def test_slab_poisson_against_float64(real_t, n):
     gs, ncomp, nranks = 2, 1, 2
     rng = np.random.default_rng(4)
     rhs = rng.uniform(size=(ncomp,) + tuple(v + 2 * gs for v in n)).astype(real_t)
-    out = _slab_solve_emulated(emu(), real_t, n, nranks, rhs, gs, ncomp)
+    out = slab_poisson_solve(_Host(), n, real_t, nranks, rhs, ncomp, backend=1)
     ref = np.zeros(rhs.shape[1:])
     UnboundedPoissonSolverOracle3D(*n, x_range=1.0, real_t=f64).solve(ref, rhs[0].astype(f64), gs)
     nzl = n[0] // nranks
@@ -203,16 +143,6 @@ def test_slab_poisson_against_float64(real_t, n):
 
 
 # -------------------------------------------------------------------------------- fused vorticity update
-def _fused_reference(w, u, gs):
-    """cross product -> curl update -> diffusion, the oracle's three sweeps in float64"""
-    ref = w.astype(f64)
-    buf = np.zeros_like(ref)
-    st.elementwise_cross_product(buf, u.astype(f64), ref)
-    st.update_vorticity_from_velocity_forcing_mpi(ref, buf, 0.3, gs)
-    st.diffusion_timestep_mpi(ref, np.zeros(ref.shape[1:]), 0.05, gs)
-    return ref
-
-
 def _fused_case(be, real_t, n, gs):
     rng = np.random.default_rng(sum(n))
     shape = tuple(v + 2 * gs for v in n)

@@ -21,12 +21,12 @@ import pytest
 import torch
 
 import bench
+from harness import _call, _free, _fused_reference, _ib_setup, _spread, cuda  # noqa: F401
 from oracle import ib as ib_oracle
 from oracle import stencils as st
 from oracle.poisson import UnboundedPoissonSolverOracle3D
 from oracle.simulator import FlowSimulatorOracle3D
 from sopht_mpi_b200 import _lib
-from test_emu_launch_coverage import _call, _Cuda, _fused_reference
 
 pytestmark = pytest.mark.gpu
 
@@ -55,18 +55,6 @@ def _rel(a, b):
 def _check(record_property, name, err, tol):
     record_property(name, err)
     assert err <= tol, (name, err)
-
-
-def _free():
-    torch.cuda.synchronize()
-    torch.cuda.empty_cache()
-
-
-@pytest.fixture(scope="module")
-def cuda():
-    if not torch.cuda.is_available():
-        pytest.skip("no CUDA device")
-    return _Cuda()
 
 
 def _inner(ncomp=0):
@@ -252,33 +240,6 @@ def test_velocity_from_stream_function(cuda, n, real_t, record_property):
 
 
 # ------------------------------------------------------------------- immersed boundary
-def _ib_setup(name):
-    """bench.py's body on its grid: the product keeps the Lagrangian arrays in the dtype of the points
-    (float64 here) on the float32 grid, with dx and the coordinate shift rounded to the grid's real_t"""
-    w = bench.workload_setup(name, bench.WORKLOADS[name][0])
-    real_t, pts = w["real_t"], w["points"]
-    assert real_t == f32 and pts.dtype == f64
-    dx = real_t(w["dx"])
-    shift = real_t(dx / 2)
-    p = _lib.IBParams()
-    p.lag_dtype, p.kernel_type, p.width = _lib.F64, 0, 2
-    p.dx, p.coord_shift = float(dx), float(shift)
-    area = w["dx"] ** 2  # the interactor's max_lag_grid_dx ** 2
-    p.stiffness, p.damping = w["k"] * area, w["c"] * area
-    g = _lib.make_grid(3, real_t, GS, w["grid"], (1,) * 6)
-    return w, g, p
-
-
-def _spread(be, g, p, forcing_lag, pos, shape):
-    """the product's spreading on one rank: scatter, then the ghost sum (which only clears the ghosts)"""
-    eul = torch.zeros(shape, dtype=torch.float32, device="cuda")
-    n = pos.shape[1]
-    _call(be, "sb200_ib_spread_owned", ctypes.byref(g), ctypes.byref(p), n, be.ptr(eul), be.ptr(forcing_lag),
-          be.ptr(pos), None, 0, None)
-    _call(be, "sb200_clear_ghost_cells", ctypes.byref(g), be.ptr(eul), 3, None)
-    return eul
-
-
 @pytest.mark.parametrize("name", ["fsi_512_f32", "rod_fsi_512x256x256_f32"])
 def test_ib_interaction_and_spreading(cuda, name, record_property):
     """sb200_ib_interact_owned (nearest index, weights, E->L interpolation, mismatch, penalty force) and

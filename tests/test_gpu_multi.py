@@ -1,30 +1,11 @@
 """Multi-GPU parity (z-slabs over NCCL): needs >= 2 visible GPUs (gpurun --gpus 2)."""
-import os
-import socket
-import subprocess
-import sys
-
 import pytest
-import torch
+
+from harness import run_ranks
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
-
-
-def _free_port():
-    s = socket.socket()
-    s.bind(("127.0.0.1", 0))
-    port = s.getsockname()[1]
-    s.close()
-    return port
 
 
 @pytest.mark.parametrize("nproc", [2, 4, 8])
 def test_slab_decomposition_against_single_domain_oracle(nproc):
-    if not torch.cuda.is_available() or torch.cuda.device_count() < nproc:
-        pytest.skip(f"needs {nproc} GPUs")
-    cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={nproc}",
-           "--master-addr", "127.0.0.1", "--master-port", str(_free_port()),
-           os.path.join(ROOT, "tests", "dist_gpu_worker.py")]
-    r = subprocess.run(cmd, capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0 and "DIST_GPU_WORKER_OK" in r.stdout, r.stdout[-3000:] + r.stderr[-5000:]
+    run_ranks("dist_gpu_worker.py", nproc, "DIST_GPU_WORKER_OK", where="gpus")

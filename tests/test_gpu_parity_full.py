@@ -24,6 +24,7 @@ import numpy as np
 import pytest
 import torch
 
+from harness import _Cuda, slab_poisson_solve
 from oracle import ib as ib_oracle
 from oracle import stencils as st
 from oracle.poisson import UnboundedPoissonSolverOracle3D
@@ -367,44 +368,6 @@ def test_peskin_weights_against_reference_golden(cuda, name):
 
 
 # ------------------------------------------------------ distributed entry points, virtual ranks
-def _virtual_slab_solve(lib, cuda, real_t, n, nranks, rhs, gs, ncomp):
-    """sb200_poisson_slab_forward / _spectral / _backward of `nranks` handles on ONE device; the
-    two all-to-alls (block q of rank r -> block r of rank q) are done here with torch copies."""
-    from sopht_mpi_b200 import _lib
-    from sopht_mpi_b200.utils.device import dptr
-
-    nz, ny, nx = n
-    nzl = nz // nranks
-    dt = torch.float32 if real_t == np.float32 else torch.float64
-    handles, send, recv, outs, locs = [], [], [], [], []
-    for r in range(nranks):
-        h = ctypes.c_void_p()
-        _lib.check(lib, lib.sb200_poisson_create(ctypes.byref(h), 3, _lib.dtype_code(real_t), nz, ny, nx, gs, 1.0,
-                                                 r, nranks, 1, None))
-        handles.append(h)
-        nel = int(lib.sb200_poisson_slab_buffer_bytes(h, ncomp)) // rhs.element_size()
-        send.append(torch.zeros(nel, dtype=dt, device=cuda))
-        recv.append(torch.zeros(nel, dtype=dt, device=cuda))
-        locs.append(rhs[:, r * nzl:r * nzl + nzl + 2 * gs].contiguous())
-        outs.append(torch.full_like(locs[-1], 7.0))
-    for r in range(nranks):
-        _lib.check(lib, lib.sb200_poisson_slab_forward(handles[r], dptr(locs[r]), ncomp, dptr(send[r]), None))
-    for r in range(nranks):
-        for q in range(nranks):
-            recv[q].view(nranks, -1)[r].copy_(send[r].view(nranks, -1)[q])
-    for r in range(nranks):
-        _lib.check(lib, lib.sb200_poisson_slab_spectral(handles[r], dptr(recv[r]), ncomp, None))
-    for r in range(nranks):
-        for q in range(nranks):
-            send[q].view(nranks, -1)[r].copy_(recv[r].view(nranks, -1)[q])
-    for r in range(nranks):
-        _lib.check(lib, lib.sb200_poisson_slab_backward(handles[r], dptr(outs[r]), ncomp, dptr(send[r]), None))
-    torch.cuda.synchronize()
-    for h in handles:
-        lib.sb200_poisson_destroy(h)
-    return outs
-
-
 @pytest.mark.parametrize("n,real_t,nranks", [((64, 32, 64), np.float32, 2), ((64, 64, 32), np.float64, 4),
                                              ((256, 256, 256), np.float32, 8), ((256, 128, 512), np.float32, 4),
                                              ((128, 128, 128), np.float64, 2)],
@@ -414,15 +377,13 @@ def test_slab_poisson_with_virtual_ranks_on_one_gpu(cuda, n, real_t, nranks):
     """SURVEY P4 (MPIDomainDoublingCommunicator3D + mpi4py-fft transposes,
     UnboundedPoissonSolverMPI3D.py:190-382) on a single GPU: the slab pipeline of every rank, with
     the transposes done by the test, must reproduce the single-domain solve."""
-    from sopht_mpi_b200 import _lib
     from sopht_mpi_b200.numeric.eulerian_grid_ops import UnboundedPoissonSolverMPI3D
 
-    lib = _lib.load()
     gs, ncomp = 2, 3
     dt = torch.float32 if real_t == np.float32 else torch.float64
     gen = torch.Generator(device=cuda).manual_seed(21)
     rhs = torch.rand((ncomp,) + tuple(v + 2 * gs for v in n), device=cuda, dtype=dt, generator=gen)
-    outs = _virtual_slab_solve(lib, cuda, real_t, n, nranks, rhs, gs, ncomp)
+    outs = slab_poisson_solve(_Cuda(), n, real_t, nranks, rhs, ncomp, backend=1)
     mc, _ = _construct(n, real_t)
     single = UnboundedPoissonSolverMPI3D(*n, mpi_construct=mc, ghost_size=gs, x_range=1.0, real_t=real_t)
     ref = torch.zeros_like(rhs)

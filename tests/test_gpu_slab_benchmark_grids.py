@@ -22,24 +22,22 @@ import ctypes
 import json
 import math
 import os
-import socket
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 import torch
 
 import bench
+from harness import _call, _free, _ib_setup, _spread, cuda, run_ranks, slab_poisson_solve, slabs  # noqa: F401
 from oracle import ib as ib_oracle
 from sopht_mpi_b200 import _lib
-from test_emu_launch_coverage import _call
-from test_gpu_benchmark_grids import GRID_256, GRID_512, GRID_ROD, GS, _free, _ib_setup, _spread, cuda  # noqa: F401
 
 pytestmark = pytest.mark.gpu
 
 f32, f64 = np.float32, np.float64
-ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
+GS = 2  # the simulator's ghost size
+GRID_512, GRID_ROD, GRID_256 = (bench.WORKLOADS[k][0] for k in ("fsi_512_f32", "rod_fsi_512x256x256_f32",
+                                                                 "vortex_ring_256_f64"))
 PS = (2, 4, 8)
 # (grid, real_t, x_range): fsi_512_f32; the rod grid (sphere_vbf_512x256x256_f32 is the same shape with
 # x_range 1.0); vortex_ring_256_f64
@@ -50,13 +48,6 @@ IB_WORKLOADS = {"512-f32": "fsi_512_f32", "256x256x512-f32-rod": "rod_fsi_512x25
 
 def _torch_t(real_t):
     return torch.float32 if real_t == f32 else torch.float64
-
-
-def _slabs(glob, nranks):
-    """each rank's slab of a padded (..., z, y, x) field: its nzl interior planes and gs ghost planes on
-    either side, filled from the neighbours (what the halo exchange leaves there)"""
-    nzl = (glob.shape[-3] - 2 * GS) // nranks
-    return [glob[..., r * nzl:r * nzl + nzl + 2 * GS, :, :].contiguous() for r in range(nranks)]
 
 
 def _rows(glob, r, nzl):
@@ -96,10 +87,6 @@ def _report(record_property, results):
     assert not bad, f"slab results differ from the single-GPU results: {bad}"
 
 
-def _ptr(t, offset_elems=0):
-    return ctypes.c_void_p(t.data_ptr() + offset_elems * t.element_size())
-
-
 # ------------------------------------------------------------------------------- Poisson
 def _single_solve(be, n, real_t, x_range, rhs, ncomp):
     sol = torch.full_like(rhs, 7.0)
@@ -111,48 +98,6 @@ def _single_solve(be, n, real_t, x_range, rhs, ncomp):
     finally:
         be.lib.sb200_poisson_destroy(h)
     return sol
-
-
-def _slab_solve(be, n, real_t, x_range, nranks, rhs, ncomp, per_component):
-    """the z-slab solve of `nranks` handles on one device.  per_component: like _solve_slabs in
-    numeric/eulerian_grid_ops/poisson.py, one forward / spectral / backward call per component with
-    ncomp = 1 at the component's offset, into exchange buffers of sb200_poisson_slab_buffer_bytes(h, 1);
-    otherwise one call of each stage with `ncomp`.  The two all-to-alls are block copies: block q of
-    rank r -> block r of rank q."""
-    locs = _slabs(rhs, nranks)
-    outs = [torch.full_like(loc, 7.0) for loc in locs]
-    vol = locs[0][0].numel() if ncomp > 1 else locs[0].numel()
-    handles = []
-    try:
-        for r in range(nranks):
-            h = ctypes.c_void_p()
-            _call(be, "sb200_poisson_create", ctypes.byref(h), 3, _lib.dtype_code(real_t), *n, GS, x_range, r, nranks,
-                  1, None)
-            handles.append(h)
-        calls = [(c, 1) for c in range(ncomp)] if per_component else [(0, ncomp)]
-        for c, k in calls:
-            nel = int(be.lib.sb200_poisson_slab_buffer_bytes(handles[0], k)) // rhs.element_size()
-            assert nel % nranks == 0
-            send = [torch.zeros(nel, dtype=rhs.dtype, device="cuda") for _ in range(nranks)]
-            recv = [torch.zeros(nel, dtype=rhs.dtype, device="cuda") for _ in range(nranks)]
-            for r in range(nranks):
-                _call(be, "sb200_poisson_slab_forward", handles[r], _ptr(locs[r], c * vol), k, be.ptr(send[r]), None)
-            for r in range(nranks):
-                for q in range(nranks):
-                    recv[q].view(nranks, -1)[r].copy_(send[r].view(nranks, -1)[q])
-            for r in range(nranks):
-                _call(be, "sb200_poisson_slab_spectral", handles[r], be.ptr(recv[r]), k, None)
-            for r in range(nranks):
-                for q in range(nranks):
-                    send[q].view(nranks, -1)[r].copy_(recv[r].view(nranks, -1)[q])
-            for r in range(nranks):
-                _call(be, "sb200_poisson_slab_backward", handles[r], _ptr(outs[r], c * vol), k, be.ptr(send[r]), None)
-            torch.cuda.synchronize()
-            del send, recv
-    finally:
-        for h in handles:
-            be.lib.sb200_poisson_destroy(h)
-    return outs
 
 
 def _ghosts_untouched(out):
@@ -177,16 +122,16 @@ def test_slab_poisson_solve_like_the_product(cuda, grid, record_property):
     results, problems = {}, []
     for nranks in PS:
         nzl = n[0] // nranks
-        outs = _slab_solve(be, n, real_t, x_range, nranks, rhs, 3, per_component=True)
+        outs = slab_poisson_solve(be, n, real_t, nranks, rhs, 3, backend=1, x_range=x_range, per_component=True)
         err = max(_mismatch(_interior_planes(o)[..., GS:-GS, GS:-GS], _rows(ref, r, nzl)[..., GS:-GS, GS:-GS])
                   for r, o in enumerate(outs))
         if not all(_ghosts_untouched(o) for o in outs):
             problems.append(f"P{nranks}: a ghost cell of the solution was written")
-        batched = _slab_solve(be, n, real_t, x_range, nranks, rhs, 3, per_component=False)
+        batched = slab_poisson_solve(be, n, real_t, nranks, rhs, 3, backend=1, x_range=x_range)
         if not all(torch.equal(a, b) for a, b in zip(outs, batched)):
             problems.append(f"P{nranks}: ncomp = 3 differs from three ncomp = 1 calls")
         del outs, batched
-        scalar = _slab_solve(be, n, real_t, x_range, nranks, rhs[1], 1, per_component=True)
+        scalar = slab_poisson_solve(be, n, real_t, nranks, rhs[1], 1, backend=1, x_range=x_range, per_component=True)
         err1 = max(_mismatch(_interior_planes(o)[..., GS:-GS, GS:-GS], _rows(ref1, r, nzl)[..., GS:-GS, GS:-GS])
                    for r, o in enumerate(scalar))
         if not all(_ghosts_untouched(o) for o in scalar):
@@ -222,7 +167,7 @@ def test_slab_fused_vorticity_update(cuda, grid, record_property):
     reach = 2 + GS
     for nranks in PS:
         nzl = n[0] // nranks
-        ws, us = _slabs(w, nranks), _slabs(u, nranks)
+        ws, us = slabs(w, nranks, GS), slabs(u, nranks, GS)
         err = 0.0
         for r in range(nranks):
             gr = _slab_grid(real_t, n, nranks, r)
@@ -273,7 +218,7 @@ def test_slab_velocity_from_stream_function(cuda, grid, record_property):
     results, problems = {}, []
     for nranks in PS:
         nzl = n[0] // nranks
-        psis, us = _slabs(psi, nranks), _slabs(u0, nranks)
+        psis, us = slabs(psi, nranks, GS), slabs(u0, nranks, GS)
         err, vmaxes = 0.0, []
         for r in range(nranks):
             gr = _slab_grid(real_t, n, nranks, r)
@@ -333,7 +278,7 @@ def test_slab_sparse_forcing_update(cuda, grid, record_property):
     record_property("body_planes", f"{zlo:.0f}-{zhi:.0f}")
     for nranks in PS:
         nzl = n[0] // nranks
-        ws, fs = _slabs(omega, nranks), _slabs(d_f, nranks)
+        ws, fs = slabs(omega, nranks, GS), slabs(d_f, nranks, GS)
         err = 0.0
         for r in range(nranks):
             gr = _slab_grid(real_t, n, nranks, r)
@@ -444,7 +389,7 @@ def test_slab_ib_interaction_and_spreading(cuda, grid, record_property):
             problems.append(f"P{nranks}: rank address differs from the oracle's")
         owners = sorted(set(own.tolist()))
         record_property(f"P{nranks}_owning_ranks", ",".join(map(str, owners)))
-        us = _slabs(eul, nranks)
+        us = slabs(eul, nranks, GS)
         total = torch.zeros_like(single)
         for r in range(nranks):
             part = interact(_slab_grid(f32, n, nranks, r), _slab_params(p, r * nzl), us[r], owner, r)
@@ -495,19 +440,15 @@ STEP_BARS = {"vorticity_field": 2e-6, "stream_func_field": 2e-6, "lag2_forcing":
              "velocity_field": 5e-6}
 
 
-def _bench_step_reference(name, path):
-    env = {k: v for k, v in os.environ.items() if k not in ("RANK", "WORLD_SIZE", "LOCAL_RANK")}
-    env.update(SB200_BENCH_STEP_WORKLOAD=name, SB200_BENCH_STEP_DIR=str(path),
-               CUDA_VISIBLE_DEVICES=os.environ.get("CUDA_VISIBLE_DEVICES", "0").split(",")[0])
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "dist_bench_step_worker.py")], env=env,
-                       capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0 and "DIST_BENCH_STEP_REFERENCE_OK" in r.stdout, r.stdout[-2000:] + r.stderr[-4000:]
+def _step_env(name, path):
+    return {"SB200_BENCH_STEP_WORKLOAD": name, "SB200_BENCH_STEP_DIR": str(path)}
 
 
 def _bench_step_single_gpu_runs(name, path):
     """the reference run, then a second single-GPU run that compares itself with it (single.json)"""
     for _ in range(2):
-        _bench_step_reference(name, path)
+        run_ranks("dist_bench_step_worker.py", 1, "DIST_BENCH_STEP_REFERENCE_OK", where="one_gpu",
+                  env=_step_env(name, path))
 
 
 def _check_bench_step(name, nranks, path, record_property):
@@ -544,27 +485,14 @@ def _check_bench_step(name, nranks, path, record_property):
 def test_bench_step_with_ranks_on_one_gpu(name, nranks, tmp_path, record_property):
     """Two steps of bench.py's step sequence as `nranks` processes on one GPU (gloo for the collectives,
     the push transport of the peer-memory exchanges) against the same steps in one process."""
-    from test_gpu_ranks_on_one_device import _run_ranks_on_one_gpu
-
-    if not torch.cuda.is_available():
-        pytest.skip("needs a GPU")
     try:
         _bench_step_single_gpu_runs(name, tmp_path)
-        _run_ranks_on_one_gpu("dist_bench_step_worker.py", nranks, "DIST_BENCH_STEP_WORKER_OK",
-                              {"SB200_TEST_SINGLE_DEVICE": "1", "SB200_PEER_WAIT_S": "300",
-                               "SB200_BENCH_STEP_WORKLOAD": name, "SB200_BENCH_STEP_DIR": str(tmp_path)})
+        run_ranks("dist_bench_step_worker.py", nranks, "DIST_BENCH_STEP_WORKER_OK", where="one_gpu",
+                  env=dict(_step_env(name, tmp_path), SB200_PEER_WAIT_S="300"))
         _check_bench_step(name, nranks, tmp_path, record_property)
     finally:
         for f in tmp_path.iterdir():  # (about 5 GB at 512^3)
             f.unlink()
-
-
-def _free_port():
-    s = socket.socket()
-    s.bind(("127.0.0.1", 0))
-    port = s.getsockname()[1]
-    s.close()
-    return port
 
 
 @pytest.mark.parametrize("name,nranks", STEP_CASES, ids=[f"{n}-P{p}" for n, p in STEP_CASES])
@@ -572,15 +500,11 @@ def test_bench_step_on_gpus(name, nranks, tmp_path, record_property):
     """The same steps with one GPU per rank under torch.distributed.run: NCCL and the default transport
     of the exchanges (the copy-engine transport on 2 and 4 ranks)."""
     if not torch.cuda.is_available() or torch.cuda.device_count() < nranks:
-        pytest.skip(f"needs {nranks} GPUs")
+        pytest.skip(f"needs {nranks} GPUs")  # before the single-GPU runs
     try:
         _bench_step_single_gpu_runs(name, tmp_path)
-        env = dict(os.environ, SB200_BENCH_STEP_WORKLOAD=name, SB200_BENCH_STEP_DIR=str(tmp_path))
-        cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={nranks}",
-               "--master-addr", "127.0.0.1", "--master-port", str(_free_port()),
-               os.path.join(ROOT, "tests", "dist_bench_step_worker.py")]
-        r = subprocess.run(cmd, env=env, capture_output=True, text=True, timeout=900)
-        assert r.returncode == 0 and "DIST_BENCH_STEP_WORKER_OK" in r.stdout, r.stdout[-3000:] + r.stderr[-5000:]
+        run_ranks("dist_bench_step_worker.py", nranks, "DIST_BENCH_STEP_WORKER_OK", where="gpus",
+                  env=_step_env(name, tmp_path))
         _check_bench_step(name, nranks, tmp_path, record_property)
     finally:
         for f in tmp_path.iterdir():

@@ -8,23 +8,18 @@
 
 Tolerances: relative L-inf <= 1e-5 (float32), <= 1e-10 (float64).
 """
-import ctypes
 import os
-import subprocess
-import sys
 import types
 
 import numpy as np
 import pytest
 import torch
 
+from harness import _Cuda, run_ranks, slab_poisson_solve
 from oracle.poisson import UnboundedPoissonSolverOracle3D
-from test_gpu_multi import _free_port
-from test_gpu_ranks_on_one_device import _run_ranks_on_one_gpu
 
 pytestmark = pytest.mark.gpu
 
-ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
 TOL = {np.float64: 1e-10, np.float32: 1e-5}
 GS = 2
 
@@ -41,47 +36,6 @@ def cuda():
 
 def _rel(a, b):
     return float((a - b).abs().max() / b.abs().max().clamp_min(1e-300))
-
-
-def _virtual_cufft_slab_solve(cuda, real_t, n, nranks, rhs, ncomp):
-    """sb200_poisson_slab_forward / _spectral / _backward of `nranks` cuFFT handles on ONE device; the two
-    all-to-alls (block q of rank r -> block r of rank q) are torch copies.  Returns each rank's padded slab."""
-    from sopht_mpi_b200 import _lib
-    from sopht_mpi_b200.utils.device import dptr
-
-    lib = _lib.load()
-    nz, ny, nx = n
-    nzl = nz // nranks
-    handles, send, recv, outs, locs = [], [], [], [], []
-    try:
-        for r in range(nranks):
-            h = ctypes.c_void_p()
-            _lib.check(lib, lib.sb200_poisson_create(ctypes.byref(h), 3, _lib.dtype_code(real_t), nz, ny, nx, GS,
-                                                     1.0, r, nranks, 0, None))
-            handles.append(h)
-            nel = int(lib.sb200_poisson_slab_buffer_bytes(h, ncomp)) // rhs.element_size()
-            send.append(torch.zeros(nel, dtype=rhs.dtype, device=cuda))
-            recv.append(torch.zeros(nel, dtype=rhs.dtype, device=cuda))
-            locs.append(rhs[:, r * nzl:r * nzl + nzl + 2 * GS].contiguous())
-            outs.append(torch.full_like(locs[-1], 7.0))
-        for r in range(nranks):
-            _lib.check(lib, lib.sb200_poisson_slab_forward(handles[r], dptr(locs[r]), ncomp, dptr(send[r]), None))
-        for r in range(nranks):
-            for q in range(nranks):
-                recv[q].view(nranks, -1)[r].copy_(send[r].view(nranks, -1)[q])
-        for r in range(nranks):
-            _lib.check(lib, lib.sb200_poisson_slab_spectral(handles[r], dptr(recv[r]), ncomp, None))
-        for r in range(nranks):
-            for q in range(nranks):
-                send[q].view(nranks, -1)[r].copy_(recv[r].view(nranks, -1)[q])
-        for r in range(nranks):
-            _lib.check(lib, lib.sb200_poisson_slab_backward(handles[r], dptr(outs[r]), ncomp, dptr(send[r]),
-                                                            None))
-        torch.cuda.synchronize()
-    finally:
-        for h in handles:
-            lib.sb200_poisson_destroy(h)
-    return outs
 
 
 def _single_rank_cufft(cuda, real_t, n, rhs):
@@ -126,7 +80,7 @@ def test_cufft_slab_solve_with_virtual_ranks(cuda, n, real_t, nranks, ncomp):
     dt = torch.float32 if real_t == np.float32 else torch.float64
     gen = torch.Generator(device=cuda).manual_seed(5)
     rhs = torch.rand((ncomp,) + tuple(v + 2 * GS for v in n), device=cuda, dtype=dt, generator=gen)
-    outs = _virtual_cufft_slab_solve(cuda, real_t, n, nranks, rhs, ncomp)
+    outs = slab_poisson_solve(_Cuda(), n, real_t, nranks, rhs, ncomp, backend=0)
     ref = _single_rank_cufft(cuda, real_t, n, rhs)
     _check_slabs(outs, ref, n, nranks, TOL[real_t])
     # and the single-rank solve is the oracle's
@@ -156,7 +110,7 @@ def test_cufft_slab_solve_at_the_refined_sphere_grid(cuda, nranks):
     del solver
     gen = torch.Generator(device=cuda).manual_seed(9)
     rhs = torch.rand((3,) + tuple(v + 2 * GS for v in n), device=cuda, dtype=torch.float32, generator=gen)
-    outs = _virtual_cufft_slab_solve(cuda, real_t, n, nranks, rhs, 3)
+    outs = slab_poisson_solve(_Cuda(), n, real_t, nranks, rhs, 3, backend=0)
     ref = _single_rank_cufft(cuda, real_t, n, rhs)
     _check_slabs(outs, ref, n, nranks, TOL[real_t])
 
@@ -181,16 +135,9 @@ def test_small_grids_stay_replicated(cuda, nranks):
 def test_cufft_slab_solve_and_steps_with_ranks_on_one_gpu(size):
     """tests/dist_slab_cufft_worker.py (vector solve and flow steps on slabs of a grid that is not a power of
     two, over the peer-memory all-to-all) with every rank a process on cuda:0"""
-    _run_ranks_on_one_gpu("dist_slab_cufft_worker.py", size, "DIST_SLAB_CUFFT_WORKER_OK",
-                          {"SB200_TEST_SINGLE_DEVICE": "1"})
+    run_ranks("dist_slab_cufft_worker.py", size, "DIST_SLAB_CUFFT_WORKER_OK", where="one_gpu")
 
 
 @pytest.mark.parametrize("nproc", [2, 3, 4, 6, 8])
 def test_cufft_slab_solve_and_steps_on_several_gpus(nproc):
-    if not torch.cuda.is_available() or torch.cuda.device_count() < nproc:
-        pytest.skip(f"needs {nproc} GPUs")
-    cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={nproc}",
-           "--master-addr", "127.0.0.1", "--master-port", str(_free_port()),
-           os.path.join(ROOT, "tests", "dist_slab_cufft_worker.py")]
-    r = subprocess.run(cmd, capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0 and "DIST_SLAB_CUFFT_WORKER_OK" in r.stdout, r.stdout[-3000:] + r.stderr[-5000:]
+    run_ranks("dist_slab_cufft_worker.py", nproc, "DIST_SLAB_CUFFT_WORKER_OK", where="gpus")

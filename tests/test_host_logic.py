@@ -1,13 +1,11 @@
 """Host-side logic: topology, halo exchange, field scatter/gather, Lagrangian rank
 ownership -- single process and world_size 2 over gloo."""
 import os
-import socket
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 
+from harness import run_ranks
 from oracle import ib as ib_oracle
 from sopht_mpi_b200.utils import (MPIConstruct2D, MPIConstruct3D, MPIGhostCommunicator3D,
                                   MPILagrangianFieldCommunicator2D, MPILagrangianFieldCommunicator3D,
@@ -117,21 +115,8 @@ def test_device_field_facade_on_cpu_tensor():
     assert np.asarray(f).sum() > 0
 
 
-def _free_port():
-    s = socket.socket()
-    s.bind(("127.0.0.1", 0))
-    port = s.getsockname()[1]
-    s.close()
-    return port
-
-
 def test_two_rank_gloo_halo_fields_and_ownership():
-    cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2",
-           "--master-addr", "127.0.0.1", "--master-port", str(_free_port()),
-           os.path.join(ROOT, "tests", "dist_worker.py")]
-    env = dict(os.environ, CUDA_VISIBLE_DEVICES="", OMP_NUM_THREADS="1")
-    r = subprocess.run(cmd, capture_output=True, text=True, timeout=600, env=env)
-    assert r.returncode == 0 and "DIST_WORKER_OK" in r.stdout, r.stdout[-3000:] + r.stderr[-3000:]
+    run_ranks("dist_worker.py", 2, "DIST_WORKER_OK", where="cpu", timeout=600)
 
 
 def test_row_block_magic_division_is_exact():
